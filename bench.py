@@ -12,7 +12,15 @@ of device slots.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]          our arm
   python bench.py --impl reference ...                          CPU restatement of the reference
+  python bench.py ... --dump-outputs DIR                        also save what the last timed step computed
 Under torchrun every rank drives one GPU with its own 1024 queries (weak scaling, no collective).
+Each GPU line (headline, packed, end to end, CROWN bounds, other workloads) times --steps steps.
+
+--dump-outputs DIR writes DIR/dense_blocks.npy (float64), the dense clique blocks that the headline loop
+(nnsdp_batch_run into the device ring) left in its ring slots after its last step: row i is query Q - n + i of
+rank 0, n = the queries of the last pass, each row the flat blocks of one query (nnsdp_batch_get_slot layout), or
+the same fixed, seeded sample of its entries when all n rows would exceed DUMP_BYTES.  The inputs depend on the
+arguments only, so two builds run with the same arguments can be compared entry for entry.
 """
 from __future__ import annotations
 
@@ -45,6 +53,7 @@ WORKLOADS = {
 }
 EXTRA_WORKLOADS = ("mid-W100-D50-beta2-Q1024", "tiny-W10-D10-beta1-Q64", "reach-W20-D10-beta2-Q64", "acas-5x50x6-beta2-Q45")
 DEFAULT_WORKLOAD = "stress-W1000-D20-beta2-Q1024"
+DUMP_BYTES = 60_000_000          # --dump-outputs: size cap of the dumped arrays (one stress query alone is 1.33 GB)
 
 
 def make_workload(name: str, rank: int, Q: int | None = None, radius_scale: float = 1.0):
@@ -130,7 +139,7 @@ def ncu_traffic(kernel):
     raise RuntimeError(f"{path} holds no launch of {kernel}: re-capture the profile (tools/ncu_summary.py)")
 
 
-def quick_measure(nb, torch, name, peak, steps=5, warmup=3):
+def quick_measure(nb, torch, name, peak, steps, warmup=3):
     """Device-timed dense and packed passes of one of the other BASELINE configs (single GPU, short)."""
     w = WORKLOADS[name]
     xdims, Ms, beta, inp = make_workload(name, 0)
@@ -170,7 +179,7 @@ def quick_measure(nb, torch, name, peak, steps=5, warmup=3):
     return out
 
 
-def crown_line(nb, torch, net, name, beta, inp, Q, steps=2):
+def crown_line(nb, torch, net, name, beta, inp, Q, steps):
     """The stress workload with the reference's DEFAULT bounds (IntervalsAutoLirpa -> CROWN on the device) instead of
     interval arithmetic: realistic bounds leave stably-active neurons in every layer, so the FP64 tensor-core Gram
     contractions (K3) run on wide layers.  Bounded sample of Q queries; packed records left in HBM."""
@@ -206,6 +215,30 @@ def crown_line(nb, torch, net, name, beta, inp, Q, steps=2):
                                        "MEASURED_PEAKS.json has no FP64 figure"}}
     b.close()
     return out
+
+
+class _DeviceDoubles:
+    """A float64 device range seen through __cuda_array_interface__, so torch can index it in place."""
+
+    def __init__(self, ptr: int, n: int):
+        self.__cuda_array_interface__ = {"shape": (n,), "typestr": "<f8", "data": (ptr, False), "strides": None,
+                                         "version": 2}
+
+
+def last_pass_outputs(torch, batch, Q: int, ring: int, nbytes: int) -> np.ndarray:
+    """The ring slots a device-only run (batch.run(None)) left behind: a pass writes queries q0 .. q0 + n - 1 into
+    slots 0 .. n - 1, so after the last pass slot i holds query Q - n + i.  Returns them as an (n, per_query) array,
+    or (n, m) with the same seeded sample of m entries per slot when n whole slots exceed `nbytes`.  Gathered on the
+    device: copying whole slots to the host would move 1.33 GB per stress query."""
+    n = Q - ring * ((Q - 1) // ring)
+    ptr, per = batch.ring_ptr()
+    batch.sync()
+    slots = torch.as_tensor(_DeviceDoubles(ptr, n * per)).view(n, per)
+    m = min(per, nbytes // (8 * n))
+    if m < per:
+        idx = np.sort(np.random.default_rng(0).choice(per, size=m, replace=False))
+        slots = slots[:, torch.from_numpy(idx).to(slots.device)]
+    return slots.cpu().numpy()
 
 
 # ------------------------------------------------------------------------------------------
@@ -438,6 +471,9 @@ def run_ours(args):
     barrier()
     ms = batch.elapsed_ms()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "dense_blocks.npy"), last_pass_outputs(torch, batch, Q, ring, DUMP_BYTES))
     stage = {k: batch.stage_ms(k) for k in ("bounds", "prepare", "gram", "emit")}  # emit = its three kernels
     ncon, nact = batch.gram_stats()
     if world > 1:
@@ -564,7 +600,7 @@ def run_ours(args):
 
     def time_e2e(flags):
         e2e_step(flags)
-        nrep = max(1, min(args.steps, 3))
+        nrep = args.steps
         if world > 1:
             dist.barrier()
         t0 = time.perf_counter()
@@ -629,8 +665,8 @@ def run_ours(args):
 
     extras, crown = None, None
     if rank == 0 and world == 1 and name == DEFAULT_WORKLOAD and not args.no_extras:
-        crown = crown_line(nb, torch, net, name, beta, inp, Q=min(Q, args.crown_queries))
-        extras = [quick_measure(nb, torch, n, peak) for n in EXTRA_WORKLOADS]
+        crown = crown_line(nb, torch, net, name, beta, inp, Q=min(Q, args.crown_queries), steps=args.steps)
+        extras = [quick_measure(nb, torch, n, peak, steps=args.steps) for n in EXTRA_WORKLOADS]
     line = None
     if rank == 0:
         # ---- CPU baseline on this box's host cores (bounded sample)
@@ -729,7 +765,13 @@ def main():
     ap.add_argument("--e2e-packed-queries", type=int, default=24)
     ap.add_argument("--radius-scale", type=float, default=1.0,
                     help="scale of the input-box radii (default 1 = BASELINE config 5); small values make every ReLU stable (Gram-heavy)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="save what the last timed step computed as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs saves the outputs of the GPU arm (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -1378,3 +1378,45 @@ def test_affine_handoff_equals_the_committed_fixture(ctx, name):
 
     for (Ck, parts, Ds), (Rk, rparts, rDs) in zip(sd.cliques_from_npz(fix), o.make_cliques(net, int(beta))):
         assert np.array_equal(Ck, Rk) and len(Ds) == len(rDs) and all(np.array_equal(a, b) for a, b in zip(Ds, rDs))
+
+
+def test_bench_dump_outputs_holds_the_last_pass(ctx, tmp_path):
+    """bench.py --dump-outputs: with 64 queries through a ring of 24 slots the last pass holds queries 48..63, and the
+    dumped rows are their clique blocks (against the oracle); a dump over the size cap is the seeded entry sample of the
+    same slots."""
+    import subprocess
+    import sys
+
+    import torch
+
+    import bench
+    import nnsdp_b200 as nb
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    name = "tiny-W10-D10-beta1-Q64"
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", name, "--ring", "24", "--steps", "2",
+                        "--no-cpu", "--no-e2e", "--no-extras", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    dump = np.load(tmp_path / "dense_blocks.npy")
+    xdims, Ms, beta, inp = bench.make_workload(name, 0)
+    net = o.FeedFwdNet(xdims, Ms)
+    cliques = o.make_cliques(net, beta)
+    assert dump.dtype == np.float64 and dump.shape == (16, sum(len(Ck) ** 2 for Ck, _, _ in cliques))
+    for i in range(16):
+        q = 48 + i
+        ref = o.run_query(net, beta, o.NumericQuery(
+            x1min=inp["x1min"][q], x1max=inp["x1max"][q], gin=inp["gamma_in"][q], gbnd=inp["gamma_bnd"][q],
+            gsec=inp["gamma_sec"][q], qc_out=o.QcSafety(S=inp["out_S"][0])))
+        for blk, rb in zip(nb.split_blocks(dump[i], cliques), ref["blocks"]):
+            assert relerr(blk, rb) <= TOL
+
+    b = nb.Batch(nb.Net(ctx, xdims, Ms), beta, Qcap=64, ring=24)
+    b.set_inputs(bench.numeric_batch(nb, name, inp), Q=64)
+    b.run(None)
+    whole = bench.last_pass_outputs(torch, b, 64, 24, bench.DUMP_BYTES)
+    sample = bench.last_pass_outputs(torch, b, 64, 24, 16 * 8 * 1000)
+    b.close()
+    assert np.array_equal(whole, dump)
+    idx = np.sort(np.random.default_rng(0).choice(whole.shape[1], size=1000, replace=False))
+    assert np.array_equal(sample, whole[:, idx])
