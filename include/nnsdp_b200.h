@@ -296,7 +296,13 @@ int32_t nnsdp_batch_set_bounds_method(nnsdp_batch* batch, int32_t method);
 /* QC diagonals, band multipliers, affine column (all queries of the batch). */
 int32_t nnsdp_batch_prepare(nnsdp_batch* batch);
 /* Gram contractions + block emission of queries [q0, q0+nq) into ring slots
- * (q - q0) % ring_queries ... ; nq <= ring_queries.  Asynchronous. */
+ * (q - q0) % ring_queries ... ; nq <= ring_queries.  Asynchronous.
+ * Ring slots are read-only to consumers.  A slot is zeroed when a pass first uses it; after that the emitter stores
+ * only the entries that can differ from what the slot already holds (structural zeros are never stored again, the
+ * diagonal block of a layer only while this query or the slot's previous one has a non-zero bulk there), and every
+ * slot still holds the complete dense output of its query after each pass.  A value written into a slot by anything
+ * but the library may therefore survive into later queries of that slot: call nnsdp_batch_ring_reset after writing
+ * into the ring. */
 int32_t nnsdp_batch_emit(nnsdp_batch* batch, int64_t q0, int64_t nq);
 /* Full pass: bounds (if the batch has no caller-supplied bounds) + prepare + emit of all
  * Q queries through the ring, chunk by chunk.  If host_out != NULL every chunk is copied
@@ -320,10 +326,13 @@ int32_t nnsdp_batch_run_ex(nnsdp_batch* batch, double* host_out, int32_t flags);
  * present; present (Q * ncells bytes, may be NULL) says which cells of each record were written.  Nothing is
  * zero-filled or scattered on the host.  flags: NNSDP_RUN_DENSE_COPY copies whole records. */
 int32_t nnsdp_batch_run_packed(nnsdp_batch* batch, double* host_records, uint8_t* present, int32_t flags);
-/* Sizes of a packed batch and, for its last run: bytes the emitter wrote, bytes moved to the host, number of
- * optional (DIAG) cells present over all queries. */
+/* Sizes of a packed batch and, for its last run: bytes the emitter stored (as nnsdp_batch_emit_stats), bytes moved to
+ * the host, number of optional (DIAG) cells present over all queries. */
 int32_t nnsdp_batch_packed_stats(nnsdp_batch* batch, int64_t* record_doubles, int64_t* ncells, int64_t* emitted_bytes,
                                  int64_t* d2h_bytes, int64_t* present_optional_cells);
+/* Bytes the emitter stored into the ring in the last nnsdp_batch_run* (every format), plus those of the
+ * nnsdp_batch_emit calls since.  Structural zeros are stored once per slot, by a memset outside this count. */
+int32_t nnsdp_batch_emit_stats(nnsdp_batch* batch, int64_t* emitted_bytes);
 /* Bytes the host gather of the last run moved: DMA (strided cells or dense), packed thin entries, and
  * bytes zero-filled by host threads; *sparse_usable = 1 if the sparse gather applies to this batch. */
 int32_t nnsdp_batch_gather_stats(nnsdp_batch* batch, int64_t* dma_bytes, int64_t* thin_bytes,
@@ -332,11 +341,16 @@ int32_t nnsdp_batch_sync(nnsdp_batch* batch);
 /* Copy results back (any pointer may be NULL). Blocking. */
 int32_t nnsdp_batch_get_bounds(nnsdp_batch* batch, double* xmin, double* xmax, double* acxmin,
                                double* acxmax, double* smin, double* smax);
+/* Copy of ring slot `slot` (read-only to consumers, see nnsdp_batch_emit). */
 int32_t nnsdp_batch_get_slot(nnsdp_batch* batch, int64_t slot, double* host_out);
 /* The affine column Z[:, a] of every query (Zdim x Q) after nnsdp_batch_prepare. */
 int32_t nnsdp_batch_get_affine(nnsdp_batch* batch, double* aff_out);
-/* Device pointer of the ring (for zero-copy consumers, e.g. torch.from_blob / CuArray). */
+/* Device pointer of the ring (for zero-copy consumers, e.g. torch.from_blob / CuArray).  The slots are read-only to
+ * consumers (see nnsdp_batch_emit). */
 int32_t nnsdp_batch_ring_ptr(nnsdp_batch* batch, uint64_t* dev_ptr, int64_t* slot_doubles);
+/* Forget what the ring slots hold: each slot is zeroed again on its next use and its next pass stores every entry.
+ * Needed only after something other than the library wrote into the ring. */
+int32_t nnsdp_batch_ring_reset(nnsdp_batch* batch);
 /* CUDA-event timing on the batch stream.  which: 0 = start, 1 = stop. */
 int32_t nnsdp_batch_event_record(nnsdp_batch* batch, int32_t which);
 int32_t nnsdp_batch_elapsed_ms(nnsdp_batch* batch, float* ms);

@@ -222,10 +222,19 @@ struct nnsdp_batch {
   DevBuf d_bands;
   DevBuf d_tmaps, d_tmap_ok;  // tensor maps of the W matrices for the TMA staging of the CR window program
   int nbands = 0, band_max_m = 0;
-  int64_t packed_emitted_bytes = 0, packed_present_cells = 0;  // of the last run
+  int64_t emitted_bytes = 0, packed_present_cells = 0;  // of the last run (emitted_bytes: what the emitter stored)
+  // Ring slot state (DESIGN.md section 4).  Slots [0, ring_zeroed) have been zeroed since creation or the last
+  // nnsdp_batch_ring_reset; structural zeros are never stored again.  slot_bulk[s * K + Br] = physical slot s holds a
+  // non-zero bulk (Gram copy, S22 Gram) in the SAME / DIAG strips of block Br.
+  int64_t ring_zeroed = 0;
+  std::vector<uint8_t> slot_bulk;
+  std::vector<int> bulk_begin;           // K + 1: the bulk strips of block Br are [bulk_begin[Br], bulk_begin[Br + 1])
+  std::vector<int64_t> bulk_entries;     // K: output entries of those strips
+  int64_t pass_entries = 0;              // entries every query of a pass stores (strips, windows, edges, band)
+  std::vector<BulkItem> sel;             // the (slot, block) pairs of the current pass
   nnsdp_sizes sz{};
   PlanHost plan;
-  DevBuf d_tiles, d_strips, d_mats, d_panel, d_goff, d_ldG;
+  DevBuf d_tiles, d_strips, d_bulk, d_mats, d_panel, d_goff, d_ldG;
   std::vector<long long> goff;
   std::vector<int> ldG;
   long long gram_per_query = 0;
@@ -288,7 +297,7 @@ struct nnsdp_batch {
     spans.clear();
   }
   std::vector<DevBuf*> all_bufs() {
-    return {&d_bands, &d_tmaps, &d_tmap_ok, &d_tiles, &d_strips, &d_mats, &d_panel, &d_goff, &d_ldG, &x1min, &x1max, &ymin, &ymax, &smin, &smax,
+    return {&d_bands, &d_tmaps, &d_tmap_ok, &d_tiles, &d_strips, &d_bulk, &d_mats, &d_panel, &d_goff, &d_ldG, &x1min, &x1max, &ymin, &ymax, &smin, &smax,
             &gin, &gbnd, &gsec, &outS, &outvec, &outinvP, &gout, &xmin, &xmax, &acxmin, &acxmax,
             &smin_c, &smax_c, &d11, &Md, &T0, &Bt, &u, &aff, &part, &act, &cnt, &Z11, &Z1K, &U,
             &gram, &ringbuf, &flags, &cr_rowsA, &cr_rowsB, &cr_bias, &cr_prel, &cr_preu, &cr_du, &cr_bu, &cr_dl};
@@ -845,8 +854,44 @@ int32_t nnsdp_batch_create(nnsdp_ctx* ctx, int32_t dev_index, const nnsdp_net* n
     NN_TRY(upload(b->d_tiles, b->plan.tiles.data(), b->plan.tiles.size() * sizeof(TileDev), b->st));
     NN_TRY(upload(b->d_mats, b->plan.mats.data(), b->plan.mats.size() * sizeof(MatDev), b->st));
     NN_TRY(b->ringbuf.ensure((size_t)b->plan.per_query_doubles * b->ring * 8));
-    NN_TRY(upload(b->d_strips, b->plan.strips.data(), b->plan.strips.size() * sizeof(StripDev), b->st));
+    b->slot_bulk.assign((size_t)b->ring * sh.K, 0);
+    // What a pass launches (the plan itself keeps every tile, ZERO included): structurally zero strips never, since a
+    // ring slot is zeroed once; in the dense formats the SAME / DIAG strips whose band is written elsewhere (every SAME
+    // strip, and the DIAG strips of wide layers) go to a per-block list, stored only for the (slot, block) pairs that
+    // need them (prepare_slots)
+    auto is_bulk = [&](const StripDev& d) {
+      return !b->packed && d.rblk >= 1 && d.rblk <= sh.K - 1 &&
+             (d.prog == PROG_SAME || (d.prog == PROG_DIAG && !b->plan.band_inline));
+    };
+    std::vector<StripDev> strips, bulk;
+    std::vector<std::vector<StripDev>> per_blk(sh.K);
+    b->pass_entries = 0;
+    b->bulk_entries.assign(sh.K, 0);
+    for (const StripDev& d : b->plan.strips) {
+      if (d.prog == PROG_ZERO) continue;
+      if (is_bulk(d)) {
+        per_blk[d.rblk].push_back(d);
+        b->bulk_entries[d.rblk] += (int64_t)d.nrows * d.ncols;
+      } else {
+        strips.push_back(d);
+        b->pass_entries += (int64_t)d.nrows * d.ncols;
+      }
+    }
+    b->bulk_begin.assign(sh.K + 1, 0);
+    for (int blk = 0; blk < sh.K; ++blk) {
+      b->bulk_begin[blk] = (int)bulk.size();
+      bulk.insert(bulk.end(), per_blk[blk].begin(), per_blk[blk].end());
+    }
+    b->bulk_begin[sh.K] = (int)bulk.size();
+    for (int i = b->plan.n_fill; i < (int)b->plan.tiles.size(); ++i)
+      b->pass_entries += (int64_t)b->plan.tiles[i].nrows * b->plan.tiles[i].ncols;
+    for (const BandDev& j : b->plan.bands)  // in-place band of the DIAG ranges: (2 beta + 1) m entries less the corners
+      if (j.ld > 0) b->pass_entries += (int64_t)j.m * (2 * beta + 1) - beta * (beta + 1);
+    NN_TRY(upload(b->d_strips, strips.data(), strips.size() * sizeof(StripDev), b->st));
+    NN_TRY(upload(b->d_bulk, bulk.data(), bulk.size() * sizeof(StripDev), b->st));
     b->pd.strips = b->d_strips.as<StripDev>();
+    b->pd.bulk = b->d_bulk.as<StripDev>();
+    b->pd.n_strips = (int)strips.size();
     b->pd.tiles = b->d_tiles.as<TileDev>();
     b->pd.mats = b->d_mats.as<MatDev>();
     b->pd.panel_desc = nullptr;
@@ -856,9 +901,12 @@ int32_t nnsdp_batch_create(nnsdp_ctx* ctx, int32_t dev_index, const nnsdp_net* n
       // emit_panel_kernel).  NNSDP_PANEL=0 keeps the two kernels.
       static const int panel_env = [] { const char* e = getenv("NNSDP_PANEL"); return e ? atoi(e) : 1; }();
       if (panel_env && !b->packed && !b->plan.panel.empty()) {
-        NN_TRY(upload(b->d_panel, b->plan.panel.data(), b->plan.panel.size() * sizeof(StripDev), b->st));
+        std::vector<StripDev> panel;
+        for (const StripDev& d : b->plan.panel)
+          if (d.prog != PROG_ZERO && (d.prog == PROG_RC || d.prog == PROG_CR || !is_bulk(d))) panel.push_back(d);
+        NN_TRY(upload(b->d_panel, panel.data(), panel.size() * sizeof(StripDev), b->st));
         b->pd.panel_desc = b->d_panel.as<StripDev>();
-        b->pd.n_panel = (int)b->plan.panel.size();
+        b->pd.n_panel = (int)panel.size();
       }
     }
     b->pd.ntiles = (int)b->plan.tiles.size();
@@ -1138,14 +1186,49 @@ int32_t nnsdp_batch_prepare(nnsdp_batch* b) {
   return NNSDP_OK;
 }
 
+// Ring slots keep what earlier passes stored in them.  A slot is zeroed the first time a pass uses it; after that the
+// SAME / DIAG strips of block Br are stored into slot s only when the query of this pass or the slot's previous query
+// has a non-zero bulk there (the Gram of a layer with a stably-active neuron; W_K' S22 W_K for Br = K-1).  Everything
+// else a pass launches is stored for every query.  The pairs to store go to b->sel; slots are physical positions in
+// the ring (dst = ring + p0 slots), queries [q0, q0 + nq) go to slots p0 .. p0 + nq - 1.
+static int32_t prepare_slots(nnsdp_batch* b, int64_t q0, int64_t nq, int64_t p0) {
+  const int64_t per = b->plan.per_query_doubles;
+  const int K = b->net->sh.K;
+  if (p0 + nq > b->ring_zeroed) {
+    NN_CUDA(cudaMemsetAsync(b->ringbuf.as<double>() + b->ring_zeroed * per, 0, (size_t)(p0 + nq - b->ring_zeroed) * per * 8,
+                            b->st));
+    std::fill(b->slot_bulk.begin() + b->ring_zeroed * K, b->slot_bulk.begin() + (p0 + nq) * K, 0);
+    b->ring_zeroed = p0 + nq;
+  }
+  b->sel.clear();
+  int64_t entries = b->pass_entries * nq;
+  for (int64_t i = 0; i < nq; ++i) {
+    const int64_t q = q0 + i;
+    uint8_t* held = &b->slot_bulk[(size_t)(p0 + i) * K];
+    for (int blk = 1; blk < K; ++blk) {
+      const int first = b->bulk_begin[blk], count = b->bulk_begin[blk + 1] - first;
+      if (count == 0) continue;
+      const bool now = blk <= K - 2 ? b->h_cnt[(size_t)q * K + blk] > 0 : b->bd.has_s22 != 0;
+      if (now || held[blk]) {
+        b->sel.push_back({(int32_t)i, first, count});
+        entries += b->bulk_entries[blk];
+      }
+      held[blk] = now;
+    }
+  }
+  if (!b->packed) b->emitted_bytes += entries * 8;
+  return NNSDP_OK;
+}
+
 // One emitter pass = fill, window and edge kernels back to back, each inside its own CUDA-event span
 // (ST_EMIT_FILL / _WINDOW / _EDGE) so that the per-kernel launch durations can be read back.
-static void emit_pass(nnsdp_batch* b, const GramDev& gd, int q0, int nq, double* dst) {
+static int32_t emit_pass(nnsdp_batch* b, const GramDev& gd, int q0, int nq, double* dst) {
   const NetPerDev& nd = *b->nd;
+  NN_TRY(prepare_slots(b, q0, nq, (dst - b->ringbuf.as<double>()) / b->plan.per_query_doubles));
   int total = 0;
   for (int which = 0; which < 3; ++which) {
     b->span_begin(ST_EMIT_FILL + which, b->st);
-    const int l = launch_emit(nd.nd, b->bd, gd, b->pd, q0, nq, dst, b->st, which);
+    const int l = launch_emit(nd.nd, b->bd, gd, b->pd, q0, nq, dst, b->st, which, b->sel.data(), (int)b->sel.size());
     b->span_end(b->st, l);
     total += l;
   }
@@ -1157,6 +1240,12 @@ static void emit_pass(nnsdp_batch* b, const GramDev& gd, int q0, int nq, double*
     total += l;
   }
   b->stage_launches[ST_EMIT] += total;
+  const cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) {
+    b->ring_zeroed = 0;  // the slots may not hold what the state says: zero them again on next use
+    return cuda_fail(e, "emitter pass", __FILE__, __LINE__);
+  }
+  return NNSDP_OK;
 }
 
 int32_t nnsdp_batch_emit(nnsdp_batch* b, int64_t q0, int64_t nq) {
@@ -1180,8 +1269,7 @@ int32_t nnsdp_batch_emit(nnsdp_batch* b, int64_t q0, int64_t nq) {
   b->span_end(b->st, l > 0 ? l : 0);
   NN_CHECK(l >= 0, NNSDP_ERR_ARG, "a hidden layer of %lld neurons is too wide for the Gram kernel's grid", (long long)b->net->max_block);
   NN_CUDA(cudaGetLastError());
-  emit_pass(b, gd, (int)q0, (int)nq, b->ringbuf.as<double>());
-  NN_CUDA(cudaGetLastError());
+  NN_TRY(emit_pass(b, gd, (int)q0, (int)nq, b->ringbuf.as<double>()));
   return NNSDP_OK;
 }
 
@@ -1323,7 +1411,7 @@ static int32_t run_impl(nnsdp_batch* b, double* host_out, uint8_t* present, int3
   const int64_t chunk = (nhalf == 2) ? b->ring / 2 : b->ring;
   const bool sparse = host_out && !b->packed && b->gp.usable && !(flags & NNSDP_RUN_DENSE_COPY);
   b->gather_bytes_dma = b->gather_bytes_zeroed = b->gather_bytes_thin = 0;
-  b->packed_emitted_bytes = b->packed_present_cells = 0;
+  b->emitted_bytes = b->packed_present_cells = 0;
   const int K = b->net->sh.K;
   const size_t ncells = b->lay.cells.size();
   // packed records: which DIAG cells a query carries is known from the Gram-active counts of prepare
@@ -1331,16 +1419,20 @@ static int32_t run_impl(nnsdp_batch* b, double* host_out, uint8_t* present, int3
     if (c.always) return true;
     return c.blk <= K - 2 ? b->h_cnt[(size_t)q * K + c.blk] > 0 : b->bd.has_s22 != 0;
   };
+  int64_t zero_entries = 0;  // structurally zero tiles of the record: zeroed once with the ring slot, never stored
+  if (b->packed)
+    for (int i = 0; i < b->plan.n_fill; ++i)
+      if (b->plan.tiles[i].prog == PROG_ZERO) zero_entries += (int64_t)b->plan.tiles[i].nrows * b->plan.tiles[i].ncols;
   if (b->packed)
     for (int64_t q = 0; q < b->Q; ++q) {
-      int64_t ent = b->lay.always_entries;
+      int64_t ent = b->lay.always_entries - zero_entries;
       for (size_t i = 0; i < ncells; ++i) {
         const PackedCell& c = b->lay.cells[i];
         const bool p = cell_present(q, c);
         if (present) present[(size_t)q * ncells + i] = p ? 1 : 0;
         if (!c.always && p) ent += b->plan.skip_absent ? b->lay.diag_entries[c.blk] : 0, ++b->packed_present_cells;
       }
-      b->packed_emitted_bytes += ent * 8;
+      b->emitted_bytes += ent * 8;
     }
   if (sparse) {
     const size_t need = (size_t)GATHER_STAGES * chunk * b->gp.thin_idx.size();
@@ -1380,7 +1472,8 @@ static int32_t run_impl(nnsdp_batch* b, double* host_out, uint8_t* present, int3
                (long long)b->net->max_block);
       NN_CUDA(cudaGetLastError());  // a failed Gram launch must not go unnoticed until the emitter has read its scratch
     }
-    emit_pass(b, gd, (int)q0, (int)nq, dst);
+    status = emit_pass(b, gd, (int)q0, (int)nq, dst);
+    if (status != NNSDP_OK) break;
     if (sparse) {
       status = gather_chunk(b, ci, q0, nq, h, dst, host_out, flags);
       used[h] = true;
@@ -1450,9 +1543,15 @@ int32_t nnsdp_batch_packed_stats(nnsdp_batch* b, int64_t* record_doubles, int64_
   NN_CHECK(b->packed, NNSDP_ERR_STATE, "the batch was not created with NNSDP_FORMAT_PACKED");
   if (record_doubles) *record_doubles = b->lay.record_doubles;
   if (ncells) *ncells = (int64_t)b->lay.cells.size();
-  if (emitted_bytes) *emitted_bytes = b->packed_emitted_bytes;
+  if (emitted_bytes) *emitted_bytes = b->emitted_bytes;
   if (d2h_bytes) *d2h_bytes = b->gather_bytes_dma;
   if (present_optional_cells) *present_optional_cells = b->packed_present_cells;
+  return NNSDP_OK;
+}
+
+int32_t nnsdp_batch_emit_stats(nnsdp_batch* b, int64_t* emitted_bytes) {
+  NN_CHECK(b && emitted_bytes, NNSDP_ERR_ARG, "NULL argument");
+  *emitted_bytes = b->emitted_bytes;
   return NNSDP_OK;
 }
 
@@ -1514,6 +1613,12 @@ int32_t nnsdp_batch_ring_ptr(nnsdp_batch* b, uint64_t* dev_ptr, int64_t* slot_do
   NN_CHECK(b != nullptr, NNSDP_ERR_ARG, "batch is NULL");
   if (dev_ptr) *dev_ptr = (uint64_t)(uintptr_t)b->ringbuf.p;
   if (slot_doubles) *slot_doubles = b->plan.per_query_doubles;
+  return NNSDP_OK;
+}
+
+int32_t nnsdp_batch_ring_reset(nnsdp_batch* b) {
+  NN_CHECK(b != nullptr, NNSDP_ERR_ARG, "batch is NULL");
+  b->ring_zeroed = 0;
   return NNSDP_OK;
 }
 

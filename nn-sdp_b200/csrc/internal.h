@@ -296,10 +296,12 @@ struct GramDev {
 };
 
 struct PlanDev {
-  const StripDev* strips;    // n_fill entries, parallel to tiles[0 .. n_fill)
+  const StripDev* strips;    // n_strips fill strips stored for every query of a pass (no ZERO strips, no bulk strips)
+  const StripDev* bulk;      // dense formats: the SAME / DIAG strips that only the (slot, block) pairs of a pass store
+  int n_strips;
   const TileDev* tiles;
   const MatDev* mats;
-  const StripDev* panel_desc;  // n_panel work items of the panel-ordered launch: fill strips as they are; window tiles re-packed
+  const StripDev* panel_desc;  // n_panel work items of the panel-ordered launch: AFF strips as they are; window tiles re-packed
                              // (prog = PROG_RC / PROG_CR, rblk, rl0 = cblk, cl0 = flags, ldG = matrix order)
   int n_panel;               // 0: fill and window kernels run one after the other
   int ntiles;                // tiles are sorted: [fill | window | edge]
@@ -358,10 +360,20 @@ int launch_prep(const NetDev& net, const BatchDev& b, int* err_flag, cudaStream_
 // pairs: npairs active (query, block) pairs (two ints each) with q0 <= query < q0 + ring slots; scratch slot = query - q0
 int launch_gram(const NetDev& net, const BatchDev& b, const GramDev& g, int max_n, int q0, const int* pairs,
                 int npairs, cudaStream_t st);
-// K4+K5: emit all tiles of queries [q0, q0+nq) to out + slot * per_query, slot = q - q0.
-// which: -1 = the whole pass (fill, window, edge kernels back to back); 0 / 1 / 2 = one of them.
+// One (slot, diagonal block) pair of a pass whose SAME / DIAG strips are stored: bulk strips [first, first + count).
+struct BulkItem {
+  int32_t slot, first, count;
+};
+constexpr int BULK_PER_LAUNCH = 512;  // pairs per launch, passed by value (6 KB of kernel parameters)
+struct BulkSel {
+  int32_t n;
+  BulkItem item[BULK_PER_LAUNCH];
+};
+// K4+K5: emit the tiles of queries [q0, q0+nq) to out + slot * per_query, slot = q - q0: every launched strip and tile
+// for every query, the bulk strips for the nsel pairs of sel.  Structural zeros are never stored.
+// which: -1 = the whole pass (fill, window, edge kernels back to back); 0 / 1 / 2 = one of them (0 holds the bulk strips).
 int launch_emit(const NetDev& net, const BatchDev& b, const GramDev& g, const PlanDev& plan,
-                int q0, int nq, double* out, cudaStream_t st, int which = -1);
+                int q0, int nq, double* out, cudaStream_t st, int which, const BulkItem* sel, int nsel);
 
 // affine-coefficient mode (kernels_affine.cu): device view of one query's QC data and of the cover
 struct AffineDev {

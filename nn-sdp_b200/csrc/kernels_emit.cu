@@ -14,7 +14,7 @@
 // PROGRAM.  One CTA runs its tile for a whole group of queries (ring slots), so whatever depends
 // on the network only -- the W tile of a window sum -- is loaded once and reused from registers /
 // shared memory for every query of the group:
-//   ZERO     structurally zero                                   -> fill
+//   ZERO     structurally zero                                   -> not stored (the ring slot is zeroed once)
 //   SAME     interior of a diagonal block (no band, no sliver)   -> copy of the Gram scratch, or fill
 //   RC       rows x_b against neurons of layer b+1               -> (2 beta+1)-tap sliding window over
 //                                                                   columns of W' held in registers
@@ -23,6 +23,8 @@
 //   GENERAL  anything (small nets, affine row/column)            -> per-entry evaluation with block lookup
 // All programs produce bit-identical values (same fma sequences, ascending neuron index).
 #include <stdlib.h>
+
+#include <algorithm>
 
 #include "internal.h"
 
@@ -460,7 +462,7 @@ __device__ __forceinline__ void emit_cr(const NetDev& net, const BatchDev& b, co
 }
 
 // ---- kernel 1: tiles whose bulk is a plain store stream; one (tile, query) per CTA -----------------
-//   ZERO  fill                 SAME  Gram copy | S22 Gram | fill
+//   SAME  Gram copy | S22 Gram | fill
 //   DIAG  SAME + the band term added to the entries with |jr - jc| <= beta as they are stored
 //   AFF   the affine row / column Z[a, :], Z[:, a]
 __device__ __forceinline__ double s22_entry(const double* WK, const double* U, int n_out, int rl, int cl) {
@@ -471,10 +473,10 @@ __device__ __forceinline__ double s22_entry(const double* WK, const double* U, i
   return acc;
 }
 
-// One strip (<= STRIP_ROWS x STRIP_COLS, or one wide affine-row job) for one query: grid = (strips, queries).
-// The 64 B descriptor is fetched with four independent 16 B loads; nothing else is looked up before the
-// first store of a ZERO strip.  Thread = row inside a TR-row chunk (x column group when the strip is
-// short); for every column the chunks start on a 32 B sector boundary of the output (rows before the strip
+// One strip (<= STRIP_ROWS x STRIP_COLS, or one wide affine-row job) for one query.  The 64 B descriptor is
+// fetched with independent 16 B loads.  Structurally zero strips are never launched: a ring slot is zeroed once
+// when it is first used and nothing else writes there (api.cu, prepare_slots).  Thread = row inside a TR-row
+// chunk (x column group when the strip is short); for every column the chunks start on a 32 B sector boundary of the output (rows before the strip
 // are masked), so each warp store covers whole sectors although ld is odd.  TR is a power of two.
 #ifndef NNSDP_FILL_MINB
 #define NNSDP_FILL_MINB 6
@@ -501,19 +503,6 @@ __device__ __forceinline__ void fill_strip(const NetDev& net, const BatchDev& b,
     int r = row0 - (int)(((size_t)(col + row0) >> 3) & 3) + tr;                       \
     if (r >= row0 && r < row_end) col[r] = (VALUE);                                   \
     for (r += TR; r < row_end; r += TR) col[r] = (VALUE);                             \
-  }
-  if (prog == PROG_ZERO) {
-    if (BAND_INLINE && nrows + 3 <= TR) {
-      // narrow layers: one (masked) row per thread and column; the kernel is issue-bound there, so the general
-      // loop's second-row handling is left out
-      for (int c = cg; c < ncols; c += ncg, col += cstep) {
-        const int r = tr - (int)(((size_t)(col + row0) >> 3) & 3);
-        if ((unsigned)r < (unsigned)nrows) col[row0 + r] = 0.0;
-      }
-      return;
-    }
-    NNSDP_STRIP_LOOP(0.0)
-    return;
   }
   const int q = q0 + slot, K = net.K;
   const int grow0 = d2.y, gcol0 = d2.z;
@@ -586,6 +575,15 @@ emit_fill_kernel(NetDev net, BatchDev b, GramDev g, PlanDev plan, int q0, int nq
   fill_strip<BAND_INLINE>(net, b, g, plan, plan.strips + blockIdx.x, blockIdx.y, q0, out);
 }
 
+// The SAME / DIAG strips of the (slot, block) pairs of `sel`: grid = (most strips of a block, pairs)
+template <bool BAND_INLINE>
+__global__ void __launch_bounds__(ETHREADS, NNSDP_FILL_MINB)
+emit_fill_kernel(NetDev net, BatchDev b, GramDev g, PlanDev plan, int q0, BulkSel sel, double* __restrict__ out) {
+  const BulkItem it = sel.item[blockIdx.y];
+  if ((int)blockIdx.x >= it.count) return;
+  fill_strip<BAND_INLINE>(net, b, g, plan, plan.bulk + it.first + blockIdx.x, it.slot, q0, out);
+}
+
 // ---- kernel 2: RC / CR window sums (128 x 32 tiles, beta <= 4) ------------------------------------
 // One kernel for both programs: their CTAs interleave in plan order, so the rows a CR tile writes and the rows the
 // RC tile of the same columns writes reach DRAM close in time (dense formats: a column of a clique block is
@@ -614,10 +612,11 @@ emit_window_kernel(NetDev net, BatchDev b, PlanDev plan, int tile0, int q0, int 
 }
 
 // ---- kernels 1 + 2 as one launch in PANEL order (dense formats of wide nets) ----------------------------------
-// A column of a clique block is written by several programs: fill strips (zero / Gram / affine pieces) and window
-// tiles.  Launched one kernel after the other, the pieces of a column reach DRAM milliseconds apart and each launch
-// covers only part of every DRAM page it touches (tools/probe_write_bw.cu: two launches 5.7 TB/s, one launch with the
-// items ordered by 32-column panel 7.0 TB/s on pure stores).  Here the work items of both kernels are sorted by
+// A column of a clique block is written by several programs: fill strips (affine pieces; the Gram pieces go out in
+// their own launch, for the (slot, block) pairs that need them) and window tiles.  Launched one kernel after the
+// other, the pieces of a column reach DRAM milliseconds apart and each launch covers only part of every DRAM page it
+// touches (tools/probe_write_bw.cu: two launches 5.7 TB/s, one launch with the items ordered by 32-column panel
+// 7.0 TB/s on pure stores).  Here the work items of both kernels are sorted by
 // (matrix, 32-column panel, row) and consecutive CTAs take consecutive items, so whole columns are written within
 // microseconds.  Inside a sub-batch of queries (see below) a window CTA writes its tile for `group` consecutive queries and
 // a strip CTA its strip for every (batch / group)-th query.
@@ -783,8 +782,29 @@ int launch_pack_thin(const double* ring, long long per_query, const long long* i
   return 1;
 }
 
+// The bulk strips of the (slot, block) pairs of one pass, BULK_PER_LAUNCH pairs per launch (kernel parameter space)
+static int launch_bulk(const NetDev& net, const BatchDev& b, const GramDev& g, const PlanDev& plan, int q0,
+                       const BulkItem* sel, int nsel, double* out, cudaStream_t st) {
+  int launches = 0;
+  for (int i0 = 0; i0 < nsel; i0 += BULK_PER_LAUNCH) {
+    BulkSel s;
+    s.n = std::min(BULK_PER_LAUNCH, nsel - i0);
+    int most = 0;
+    for (int i = 0; i < s.n; ++i) {
+      s.item[i] = sel[i0 + i];
+      most = std::max(most, s.item[i].count);
+    }
+    if (most == 0) continue;
+    const dim3 grid((unsigned)most, (unsigned)s.n);
+    if (plan.band_inline) emit_fill_kernel<true><<<grid, ETHREADS, 0, st>>>(net, b, g, plan, q0, s, out);
+    else emit_fill_kernel<false><<<grid, ETHREADS, 0, st>>>(net, b, g, plan, q0, s, out);
+    ++launches;
+  }
+  return launches;
+}
+
 int launch_emit(const NetDev& net, const BatchDev& b, const GramDev& g, const PlanDev& plan,
-                int q0, int nq, double* out, cudaStream_t st, int which) {
+                int q0, int nq, double* out, cudaStream_t st, int which, const BulkItem* sel, int nsel) {
   if (nq <= 0) return 0;
   static const int wgroup = [] { const char* e = getenv("NNSDP_WINDOW_GROUP"); int v = e ? atoi(e) : 4; return v < 1 ? 1 : (v > SLOT_GROUP ? SLOT_GROUP : v); }();
   // queries per edge CTA: one when a pass holds few queries (wide nets, 8 ring slots), eight when it holds many
@@ -812,9 +832,9 @@ int launch_emit(const NetDev& net, const BatchDev& b, const GramDev& g, const Pl
       ++launches;
     }
   } else {
-  if (plan.n_fill > 0 && (which < 0 || which == 0)) {
-    if (plan.band_inline) emit_fill_kernel<true><<<dim3(plan.n_fill, nq), ETHREADS, 0, st>>>(net, b, g, plan, q0, nq, out);
-    else emit_fill_kernel<false><<<dim3(plan.n_fill, nq), ETHREADS, 0, st>>>(net, b, g, plan, q0, nq, out);
+  if (plan.n_strips > 0 && (which < 0 || which == 0)) {
+    if (plan.band_inline) emit_fill_kernel<true><<<dim3(plan.n_strips, nq), ETHREADS, 0, st>>>(net, b, g, plan, q0, nq, out);
+    else emit_fill_kernel<false><<<dim3(plan.n_strips, nq), ETHREADS, 0, st>>>(net, b, g, plan, q0, nq, out);
     ++launches;
   }
   if (plan.n_window > 0 && (which < 0 || which == 1)) {
@@ -836,6 +856,7 @@ int launch_emit(const NetDev& net, const BatchDev& b, const GramDev& g, const Pl
     ++launches;
   }
   }
+  if (which < 0 || which == 0) launches += launch_bulk(net, b, g, plan, q0, sel, nsel, out, st);
   if (plan.n_edge > 0 && (which < 0 || which == 2)) {
     emit_edge_kernel<<<dim3(plan.n_edge, (nq + egroup - 1) / egroup), ETHREADS, 0, st>>>(
         net, b, g, plan, plan.n_fill + plan.n_window, q0, nq, egroup, out);

@@ -117,6 +117,8 @@ PROTOTYPES = {
     "nnsdp_batch_get_slot": (c_i32, [c_vp, c_i64, c_dp]),
     "nnsdp_batch_get_affine": (c_i32, [c_vp, c_dp]),
     "nnsdp_batch_ring_ptr": (c_i32, [c_vp, C.POINTER(c_u64), C.POINTER(c_i64)]),
+    "nnsdp_batch_ring_reset": (c_i32, [c_vp]),
+    "nnsdp_batch_emit_stats": (c_i32, [c_vp, c_i64p]),
     "nnsdp_batch_event_record": (c_i32, [c_vp, c_i32]),
     "nnsdp_batch_elapsed_ms": (c_i32, [c_vp, C.POINTER(C.c_float)]),
     "nnsdp_batch_stage_ms": (c_i32, [c_vp, c_i32, C.POINTER(C.c_float), C.POINTER(c_i64)]),

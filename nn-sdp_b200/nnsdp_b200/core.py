@@ -566,6 +566,16 @@ class Batch:
         L.check(L.lib.nnsdp_batch_ring_ptr(self._h, C.byref(p), C.byref(n)))
         return int(p.value), int(n.value)
 
+    def emitted_bytes(self) -> int:
+        """nnsdp_batch_emit_stats: bytes the emitter stored in the last run (+ emit calls since), every format."""
+        v = L.c_i64(0)
+        L.check(L.lib.nnsdp_batch_emit_stats(self._h, C.byref(v)))
+        return int(v.value)
+
+    def ring_reset(self):
+        """nnsdp_batch_ring_reset: zero every ring slot again on its next use (after writing into the ring)."""
+        L.check(L.lib.nnsdp_batch_ring_reset(self._h))
+
     def event_record(self, which: int):
         L.check(L.lib.nnsdp_batch_event_record(self._h, which))
 
