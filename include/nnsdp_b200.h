@@ -408,6 +408,41 @@ int32_t nnsdp_affine_get(nnsdp_affine* affine, int64_t* ent_row, int64_t* ent_co
                          int64_t* coo_ent, int64_t* coo_var, double* coo_val);
 int32_t nnsdp_affine_destroy(nnsdp_affine* affine);
 
+/* Batched affine-coefficient mode: the forms of Q queries in one call -- the directions of a reach polytope
+ * (src/NnSdp.jl:73-95) or the members of a vnnlib property (experiments/vnnlib_utils.jl:58-74).  Same meaning as
+ * nnsdp_affine_create, per query q:
+ *   Z_q[ent_row[e], ent_col[e]](gamma) = z0[q * nent + e] + (A_{group_of[q]} gamma)[e]
+ * with one out_kind (so one variable layout) for the batch.  Multipliers in `in` are ignored; bounds are the caller's
+ * when in->ymin != NULL, IBP from the box otherwise.
+ *   groups: the coefficients depend only on x1min, x1max and, when supplied, ymin, ymax, smin, smax.  Queries with
+ *     equal bytes in those columns form one group (numbered in order of first appearance) and share one matrix A_g;
+ *     a stride of 0 shares the column.  z0 depends on the output QC and is computed for every query.
+ *   A_g (nent x nvar) is canonical CSC: var_ptr[nvar + 1] (1-based, var_ptr[0] = 1), ent_idx (1-based entries,
+ *     strictly ascending within a variable), val; duplicate (entry, variable) pairs of the COO form are summed in the
+ *     order nnsdp_affine_get lists them, explicit zeros are kept.  Julia: SparseMatrixCSC(nent, nvar, var_ptr,
+ *     ent_idx, val); scipy: csc_matrix((val, ent_idx - 1, var_ptr - 1), shape = (nent, nvar)).
+ * The call runs on the context's first device with a working batch of the network's idle-batch cache; the handle
+ * holds only the results.  NNSDP_ERR_NOMEM when max_nnz > 0 and a group has more than max_nnz coefficients (the
+ * message names the group); NNSDP_ERR_ARG for Q < 1, a group out of range, a NULL handle (destroy accepts NULL).
+ * Output pointers of the getters may be NULL. */
+typedef struct nnsdp_affine_batch nnsdp_affine_batch;
+typedef struct {
+  int64_t Q, ngroups;
+  int64_t nvar, nent;                          /* shared by every query: one out_kind per batch        */
+  int64_t var_in, var_out, var_bnd, var_sec;   /* as nnsdp_affine_sizes                               */
+  int64_t nnz_total, nnz_max;                  /* merged coefficients over all groups / largest group */
+} nnsdp_affine_batch_sizes;
+int32_t nnsdp_affine_create_batch(nnsdp_ctx* ctx, const nnsdp_net* net, int64_t beta, int64_t Q,
+                                  const nnsdp_query_inputs* in, int64_t max_nnz,
+                                  nnsdp_affine_batch** h, nnsdp_affine_batch_sizes* sizes);
+/* group_of[Q]: 0-based group of every query; group_nnz[ngroups]; group_first[ngroups]: first query of each group */
+int32_t nnsdp_affine_batch_groups(nnsdp_affine_batch* h, int64_t* group_of, int64_t* group_nnz, int64_t* group_first);
+/* entry positions (1-based, as nnsdp_affine_get) and z0 of every query: z0[q * nent + e] */
+int32_t nnsdp_affine_batch_get(nnsdp_affine_batch* h, int64_t* ent_row, int64_t* ent_col, double* z0);
+/* A_g of group g as CSC: var_ptr[nvar + 1], ent_idx[nnz_g], val[nnz_g] */
+int32_t nnsdp_affine_batch_get_group(nnsdp_affine_batch* h, int64_t g, int64_t* var_ptr, int64_t* ent_idx, double* val);
+int32_t nnsdp_affine_batch_destroy(nnsdp_affine_batch* h);
+
 #ifdef __cplusplus
 }
 #endif

@@ -14,6 +14,7 @@
 #include <memory>
 #include <mutex>
 #include <thread>
+#include <unordered_map>
 
 #include <cuda.h>  // CUtensorMap and its enums; cuTensorMapEncodeTiled is obtained through cudaGetDriverEntryPoint
 
@@ -376,7 +377,7 @@ int32_t check_flags(nnsdp_batch* b, const char* where) {
 extern "C" {
 
 const char* nnsdp_last_error(void) { return g_err.c_str(); }
-int32_t nnsdp_version(void) { return 100; }
+int32_t nnsdp_version(void) { return 101; }
 
 int32_t nnsdp_device_count(int32_t* count) {
   NN_CHECK(count != nullptr, NNSDP_ERR_ARG, "count is NULL");
@@ -2407,6 +2408,54 @@ struct nnsdp_affine {
   DevBuf d_lo, d_colptr, d_counts, d_offs, d_ent, d_var, d_val, d_z0;
 };
 
+namespace {
+
+// The cover of the cliques: column c holds rows [lo(c), c]; lo(c) = smallest index sharing a clique with c.
+// col_ptr[c] = first entry of column c (upper triangle, column-major), col_ptr[Zdim] = nent.
+int32_t affine_cover(const Shape& sh, int64_t beta, std::vector<int>* lo, std::vector<long long>* col_ptr) {
+  CliqueInfoHost ci;
+  NN_TRY(make_cliques_host(sh, beta, &ci));
+  lo->assign((size_t)sh.Zdim, 0);
+  for (int64_t c = 0; c < sh.Zdim; ++c) {
+    int64_t l = c;
+    for (const CliqueRanges& ck : ci.ck) {
+      bool has = false;
+      for (int s = 0; s < ck.nseg; ++s) has |= (c >= ck.lo[s] && c <= ck.hi[s]);
+      if (has) l = std::min(l, ck.lo[0]);
+    }
+    (*lo)[c] = (int)l;
+  }
+  col_ptr->assign((size_t)sh.Zdim + 1, 0);
+  for (int64_t c = 0; c < sh.Zdim; ++c) (*col_ptr)[c + 1] = (*col_ptr)[c] + (c - (*lo)[c] + 1);
+  return NNSDP_OK;
+}
+
+// 1-based (row, column) of every cover entry
+void cover_entries(const std::vector<int>& lo, const std::vector<long long>& col_ptr, int64_t* ent_row, int64_t* ent_col) {
+  if (!ent_row && !ent_col) return;
+  for (int64_t c = 0; c + 1 < (int64_t)col_ptr.size(); ++c)
+    for (int64_t r = lo[c]; r <= c; ++r) {
+      const int64_t e = col_ptr[c] + (r - lo[c]);
+      if (ent_row) ent_row[e] = r + 1;  // 1-based on the wire
+      if (ent_col) ent_col[e] = c + 1;
+    }
+}
+
+// The query with every multiplier zero (stride 0): the prepared vectors then hold the constant part of Z.
+// zeros must hold max(secdim, 1) doubles, zero1 one.
+nnsdp_query_inputs zero_multipliers(const nnsdp_query_inputs& in, const double* zeros, const double* zero1) {
+  nnsdp_query_inputs q = in;
+  q.gamma_in = q.gamma_bnd = q.gamma_sec = zeros;
+  q.gamma_in_stride = q.gamma_bnd_stride = q.gamma_sec_stride = 0;
+  if (q.out_kind != NNSDP_OUT_SAFETY) {
+    q.gamma_out = zero1;
+    q.gamma_out_stride = 0;
+  }
+  return q;
+}
+
+}  // namespace
+
 extern "C" {
 
 int32_t nnsdp_affine_destroy(nnsdp_affine* h) {
@@ -2434,36 +2483,14 @@ int32_t nnsdp_affine_create(nnsdp_ctx* ctx, const nnsdp_net* net, int64_t beta,
   NN_TRY(nnsdp_batch_create(ctx, 0, net, beta, 1, 1, 0, &h->batch));
   nnsdp_batch* b = h->batch;
   // one query with every multiplier zero: the prepared vectors then hold the constant part of Z
-  nnsdp_query_inputs q = *in;
   std::vector<double> zeros((size_t)std::max<int64_t>(b->sz.secdim, 1), 0.0);
   const double zero1 = 0.0;
-  q.gamma_in = zeros.data();
-  q.gamma_bnd = zeros.data();
-  q.gamma_sec = zeros.data();
-  q.gamma_in_stride = q.gamma_bnd_stride = q.gamma_sec_stride = 0;
-  if (q.out_kind != NNSDP_OUT_SAFETY) {
-    q.gamma_out = &zero1;
-    q.gamma_out_stride = 0;
-  }
+  const nnsdp_query_inputs q = zero_multipliers(*in, zeros.data(), &zero1);
   NN_TRY(nnsdp_batch_set_inputs(b, 1, &q));
   if (!b->bounds_supplied) NN_TRY(nnsdp_batch_bounds(b));
   NN_TRY(nnsdp_batch_prepare(b));
   NN_CUDA(cudaSetDevice(b->dev));
-  // cover: column c holds rows [lo(c), c]; lo(c) = smallest index sharing a clique with c
-  CliqueInfoHost ci;
-  NN_TRY(make_cliques_host(sh, beta, &ci));
-  h->lo.assign((size_t)sh.Zdim, 0);
-  for (int64_t c = 0; c < sh.Zdim; ++c) {
-    int64_t lo = c;
-    for (const CliqueRanges& ck : ci.ck) {
-      bool has = false;
-      for (int s = 0; s < ck.nseg; ++s) has |= (c >= ck.lo[s] && c <= ck.hi[s]);
-      if (has) lo = std::min(lo, ck.lo[0]);
-    }
-    h->lo[c] = (int)lo;
-  }
-  h->col_ptr.assign((size_t)sh.Zdim + 1, 0);
-  for (int64_t c = 0; c < sh.Zdim; ++c) h->col_ptr[c + 1] = h->col_ptr[c] + (c - h->lo[c] + 1);
+  NN_TRY(affine_cover(sh, beta, &h->lo, &h->col_ptr));
   nnsdp_affine_sizes& sz = h->sz;
   sz.var_in = 0;
   sz.var_out = sh.n_in();
@@ -2509,7 +2536,7 @@ int32_t nnsdp_affine_create(nnsdp_ctx* ctx, const nnsdp_net* net, int64_t beta,
   NN_TRY(h->d_z0.ensure((size_t)std::max<int64_t>(sz.nent, 1) * 8));
   launch_affine_fill(nd, A, h->d_offs.as<long long>(), h->d_ent.as<long long>(), h->d_var.as<long long>(),
                      h->d_val.as<double>(), b->st);
-  launch_affine_z0(nd, b->bd, A, h->d_z0.as<double>(), b->st);
+  launch_affine_z0(nd, b->bd, A, sz.nent, 1, h->d_z0.as<double>(), b->st);
   NN_CUDA(cudaGetLastError());
   NN_CUDA(cudaStreamSynchronize(b->st));
   guard.h = nullptr;
@@ -2522,14 +2549,8 @@ int32_t nnsdp_affine_get(nnsdp_affine* h, int64_t* ent_row, int64_t* ent_col, do
   NN_CHECK(h != nullptr, NNSDP_ERR_ARG, "affine handle is NULL");
   nnsdp_batch* b = h->batch;
   NN_CUDA(cudaSetDevice(b->dev));
-  const int64_t Zdim = b->net->sh.Zdim, nnz = h->sz.nnz;
-  if (ent_row || ent_col)
-    for (int64_t c = 0; c < Zdim; ++c)
-      for (int64_t r = h->lo[c]; r <= c; ++r) {
-        const int64_t e = h->col_ptr[c] + (r - h->lo[c]);
-        if (ent_row) ent_row[e] = r + 1;  // 1-based on the wire
-        if (ent_col) ent_col[e] = c + 1;
-      }
+  const int64_t nnz = h->sz.nnz;
+  cover_entries(h->lo, h->col_ptr, ent_row, ent_col);
   if (z0) NN_CUDA(cudaMemcpyAsync(z0, h->d_z0.p, (size_t)h->sz.nent * 8, cudaMemcpyDeviceToHost, b->st));
   if (coo_ent && nnz) NN_CUDA(cudaMemcpyAsync(coo_ent, h->d_ent.p, (size_t)nnz * 8, cudaMemcpyDeviceToHost, b->st));
   if (coo_var && nnz) NN_CUDA(cudaMemcpyAsync(coo_var, h->d_var.p, (size_t)nnz * 8, cudaMemcpyDeviceToHost, b->st));
@@ -2539,6 +2560,237 @@ int32_t nnsdp_affine_get(nnsdp_affine* h, int64_t* ent_row, int64_t* ent_col, do
     for (int64_t i = 0; i < nnz; ++i) coo_ent[i] += 1;
   if (coo_var)
     for (int64_t i = 0; i < nnz; ++i) coo_var[i] += 1;
+  return NNSDP_OK;
+}
+
+}  // extern "C"
+
+// -----------------------------------------------------------------------------------------
+// batched affine-coefficient mode: one call for the queries of a reach polytope or a vnnlib property.  Queries whose
+// coefficients are equal (same box, and same caller bounds when supplied) form a group that shares one canonical CSC
+// matrix; z0 is per query.
+// -----------------------------------------------------------------------------------------
+struct nnsdp_affine_batch {
+  int dev = 0;
+  nnsdp_affine_batch_sizes sz{};
+  std::vector<int> lo;                   // the cover, as in nnsdp_affine
+  std::vector<long long> col_ptr;
+  std::vector<int64_t> group_of, group_first;
+  std::vector<long long> group_start;    // ngroups + 1: first coefficient of every group in d_ent / d_val
+  DevBuf d_offs;                         // ngroups * nvar + 1: first coefficient of (group, variable)
+  DevBuf d_ent, d_val, d_z0;             // 0-based entries, values; z0 (Q x nent)
+};
+
+namespace {
+
+// Groups queries by the bytes of the columns the coefficients depend on: the box, and the bounds when the caller
+// supplies them.  Columns with stride 0 are the same for every query.  Groups are numbered in order of first
+// appearance.
+void group_queries(const nnsdp_query_inputs& in, int64_t Q, int64_t n_in, int64_t acdim, std::vector<int64_t>* group_of,
+                   std::vector<int64_t>* first) {
+  struct Col {
+    const double* p;
+    int64_t stride, len;
+  };
+  std::vector<Col> cols;
+  auto add = [&](const double* p, int64_t stride, int64_t len) {
+    if (p && stride != 0 && len > 0) cols.push_back({p, stride, len});
+  };
+  add(in.x1min, in.x1min_stride, n_in);
+  add(in.x1max, in.x1max_stride, n_in);
+  if (in.ymin) {
+    add(in.ymin, in.ymin_stride, acdim);
+    add(in.ymax, in.ymax_stride, acdim);
+    add(in.smin, in.smin_stride, acdim);
+    add(in.smax, in.smax_stride, acdim);
+  }
+  auto hash = [&](int64_t q) {
+    uint64_t h = 1469598103934665603ull;
+    for (const Col& c : cols) {
+      const double* x = c.p + q * c.stride;
+      for (int64_t i = 0; i < c.len; ++i) {
+        uint64_t w;
+        memcpy(&w, x + i, 8);
+        h = (h ^ w) * 1099511628211ull;
+        h ^= h >> 29;
+      }
+    }
+    return h;
+  };
+  auto same = [&](int64_t q, int64_t r) {
+    for (const Col& c : cols)
+      if (memcmp(c.p + q * c.stride, c.p + r * c.stride, (size_t)c.len * 8) != 0) return false;
+    return true;
+  };
+  group_of->assign((size_t)Q, 0);
+  first->clear();
+  std::unordered_map<uint64_t, std::vector<int64_t>> by_hash;  // hash -> groups
+  for (int64_t q = 0; q < Q; ++q) {
+    std::vector<int64_t>& gs = by_hash[hash(q)];
+    int64_t g = -1;
+    for (int64_t c : gs)
+      if (same(q, (*first)[c])) { g = c; break; }
+    if (g < 0) {
+      g = (int64_t)first->size();
+      first->push_back(q);
+      gs.push_back(g);
+    }
+    (*group_of)[q] = g;
+  }
+}
+
+}  // namespace
+
+extern "C" {
+
+int32_t nnsdp_affine_batch_destroy(nnsdp_affine_batch* h) {
+  if (!h) return NNSDP_OK;
+  cudaSetDevice(h->dev);
+  for (DevBuf* x : {&h->d_offs, &h->d_ent, &h->d_val, &h->d_z0}) x->release();
+  delete h;
+  return NNSDP_OK;
+}
+
+int32_t nnsdp_affine_create_batch(nnsdp_ctx* ctx, const nnsdp_net* net, int64_t beta, int64_t Q,
+                                  const nnsdp_query_inputs* in, int64_t max_nnz, nnsdp_affine_batch** out,
+                                  nnsdp_affine_batch_sizes* sizes) {
+  NN_CHECK(out != nullptr, NNSDP_ERR_ARG, "affine batch output pointer is NULL");
+  *out = nullptr;
+  NN_CHECK(ctx && net && in && sizes, NNSDP_ERR_ARG, "NULL argument");
+  NN_CHECK(Q >= 1, NNSDP_ERR_ARG, "Q must be >= 1");
+  const Shape& sh = net->sh;
+  nnsdp_affine_batch* h = new nnsdp_affine_batch();
+  struct Guard {
+    nnsdp_affine_batch* h;
+    ~Guard() { if (h) nnsdp_affine_batch_destroy(h); }
+  } guard{h};
+  // scratch of this call, released on every return (declared before the batch holder: the holder hands the batch
+  // back first, after the stream has been synchronised or an error left it)
+  DevBuf d_lo, d_colptr, d_first, d_sums, d_starts;
+  struct Rel {
+    DevBuf* bufs[5];
+    ~Rel() { for (DevBuf* x : bufs) x->release(); }
+  } rel{{&d_lo, &d_colptr, &d_first, &d_sums, &d_starts}};
+  // the working batch (bounds, prepared constant part) comes from the network's cache and goes back on return
+  BatchHolder holder;
+  NN_TRY(holder.acquire(ctx, 0, net, beta, Q, 1, 0));
+  nnsdp_batch* b = holder.b;
+  h->dev = b->dev;
+  std::vector<double> zeros((size_t)std::max<int64_t>(b->sz.secdim, 1), 0.0);
+  const double zero1 = 0.0;
+  const nnsdp_query_inputs q = zero_multipliers(*in, zeros.data(), &zero1);
+  NN_TRY(nnsdp_batch_set_inputs(b, Q, &q));
+  if (!b->bounds_supplied) NN_TRY(nnsdp_batch_bounds(b));
+  NN_TRY(nnsdp_batch_prepare(b));
+  NN_CUDA(cudaSetDevice(b->dev));
+  cudaStream_t st = b->st;
+  group_queries(*in, Q, sh.n_in(), sh.acdim, &h->group_of, &h->group_first);
+  const int64_t G = (int64_t)h->group_first.size();
+  NN_TRY(affine_cover(sh, beta, &h->lo, &h->col_ptr));
+  nnsdp_affine_batch_sizes& sz = h->sz;
+  sz.Q = Q;
+  sz.ngroups = G;
+  sz.var_in = 0;
+  sz.var_out = sh.n_in();
+  sz.var_bnd = sz.var_out + (in->out_kind == NNSDP_OUT_SAFETY ? 0 : 1);
+  sz.var_sec = sz.var_bnd + sh.acdim;
+  sz.nvar = sz.var_sec + b->sz.secdim;
+  sz.nent = h->col_ptr[sh.Zdim];
+  NN_TRY(upload(d_lo, h->lo.data(), h->lo.size() * 4, st));
+  NN_TRY(upload(d_colptr, h->col_ptr.data(), h->col_ptr.size() * 8, st));
+  NN_TRY(upload(d_first, h->group_first.data(), (size_t)G * 8, st));
+  const BatchDev& bd = b->bd;
+  AffineDev A{};
+  A.nvar = sz.nvar;
+  A.var_out = sz.var_out;
+  A.var_bnd = sz.var_bnd;
+  A.var_sec = sz.var_sec;
+  A.acdim = sh.acdim;
+  A.lamdim = b->sz.lamdim;
+  A.beta = beta;
+  A.out_kind = in->out_kind;
+  A.x1min = bd.x1min, A.s_x1min = bd.s_x1min;
+  A.x1max = bd.x1max, A.s_x1max = bd.s_x1max;
+  A.ymin = bd.ymin, A.s_ymin = bd.s_ymin;
+  A.ymax = bd.ymax, A.s_ymax = bd.s_ymax;
+  A.smin = bd.smin, A.s_smin = bd.s_smin;
+  A.smax = bd.smax, A.s_smax = bd.s_smax;
+  A.col_ptr = d_colptr.as<long long>();
+  A.lo = d_lo.as<int>();
+  const NetDev& nd = b->nd->nd;
+  // merged counts per (group, variable) -> exclusive scan on the device -> group starts: one small copy to the host
+  const int64_t N = G * sz.nvar + 1;
+  NN_TRY(h->d_offs.ensure((size_t)N * 8));
+  long long* offs = h->d_offs.as<long long>();
+  NN_CUDA(cudaMemsetAsync(offs + (N - 1), 0, 8, st));
+  launch_affine_csc_count(nd, A, d_first.as<long long>(), G, offs, st);
+  NN_TRY(d_sums.ensure((size_t)scan_scratch_len(N) * 8));
+  launch_scan_exclusive(offs, N, d_sums.as<long long>(), st);
+  NN_TRY(d_starts.ensure((size_t)(G + 1) * 8));
+  launch_affine_group_starts(offs, sz.nvar, G, d_starts.as<long long>(), st);
+  NN_CUDA(cudaGetLastError());
+  h->group_start.resize((size_t)G + 1);
+  NN_CUDA(cudaMemcpyAsync(h->group_start.data(), d_starts.p, (size_t)(G + 1) * 8, cudaMemcpyDeviceToHost, st));
+  NN_CUDA(cudaStreamSynchronize(st));
+  sz.nnz_total = h->group_start[G];
+  sz.nnz_max = 0;
+  int64_t worst = 0;
+  for (int64_t g = 0; g < G; ++g) {
+    const int64_t n = h->group_start[g + 1] - h->group_start[g];
+    if (n > sz.nnz_max) sz.nnz_max = n, worst = g;
+  }
+  *sizes = sz;
+  NN_CHECK(max_nnz <= 0 || sz.nnz_max <= max_nnz, NNSDP_ERR_NOMEM,
+           "affine group %lld (first query %lld) has %lld coefficients, more than max_nnz = %lld (the Gram term is "
+           "n_k^2 per stably-active neuron: wide layers need the factored form)",
+           (long long)worst, (long long)h->group_first[worst], (long long)sz.nnz_max, (long long)max_nnz);
+  NN_TRY(h->d_ent.ensure((size_t)std::max<int64_t>(sz.nnz_total, 1) * 8));
+  NN_TRY(h->d_val.ensure((size_t)std::max<int64_t>(sz.nnz_total, 1) * 8));
+  NN_TRY(h->d_z0.ensure((size_t)std::max<int64_t>(Q * sz.nent, 1) * 8));
+  launch_affine_csc_fill(nd, A, d_first.as<long long>(), G, offs, h->d_ent.as<long long>(), h->d_val.as<double>(), st);
+  launch_affine_z0(nd, bd, A, sz.nent, (int)Q, h->d_z0.as<double>(), st);
+  NN_CUDA(cudaGetLastError());
+  NN_CUDA(cudaStreamSynchronize(st));
+  guard.h = nullptr;
+  *out = h;
+  return NNSDP_OK;
+}
+
+int32_t nnsdp_affine_batch_groups(nnsdp_affine_batch* h, int64_t* group_of, int64_t* group_nnz, int64_t* group_first) {
+  NN_CHECK(h != nullptr, NNSDP_ERR_ARG, "affine batch handle is NULL");
+  const int64_t G = h->sz.ngroups;
+  if (group_of) memcpy(group_of, h->group_of.data(), h->group_of.size() * 8);
+  if (group_first) memcpy(group_first, h->group_first.data(), (size_t)G * 8);
+  if (group_nnz)
+    for (int64_t g = 0; g < G; ++g) group_nnz[g] = h->group_start[g + 1] - h->group_start[g];
+  return NNSDP_OK;
+}
+
+int32_t nnsdp_affine_batch_get(nnsdp_affine_batch* h, int64_t* ent_row, int64_t* ent_col, double* z0) {
+  NN_CHECK(h != nullptr, NNSDP_ERR_ARG, "affine batch handle is NULL");
+  cover_entries(h->lo, h->col_ptr, ent_row, ent_col);
+  if (z0) {
+    NN_CUDA(cudaSetDevice(h->dev));
+    NN_CUDA(cudaMemcpy(z0, h->d_z0.p, (size_t)(h->sz.Q * h->sz.nent) * 8, cudaMemcpyDeviceToHost));
+  }
+  return NNSDP_OK;
+}
+
+int32_t nnsdp_affine_batch_get_group(nnsdp_affine_batch* h, int64_t g, int64_t* var_ptr, int64_t* ent_idx, double* val) {
+  NN_CHECK(h != nullptr, NNSDP_ERR_ARG, "affine batch handle is NULL");
+  NN_CHECK(g >= 0 && g < h->sz.ngroups, NNSDP_ERR_ARG, "group %lld outside [0, %lld)", (long long)g,
+           (long long)h->sz.ngroups);
+  NN_CUDA(cudaSetDevice(h->dev));
+  const int64_t nvar = h->sz.nvar, s0 = h->group_start[g], nnz = h->group_start[g + 1] - s0;
+  if (var_ptr) {
+    NN_CUDA(cudaMemcpy(var_ptr, h->d_offs.as<long long>() + g * nvar, (size_t)(nvar + 1) * 8, cudaMemcpyDeviceToHost));
+    for (int64_t v = 0; v <= nvar; ++v) var_ptr[v] = var_ptr[v] - s0 + 1;  // 1-based on the wire
+  }
+  if (ent_idx && nnz) {
+    NN_CUDA(cudaMemcpy(ent_idx, h->d_ent.as<long long>() + s0, (size_t)nnz * 8, cudaMemcpyDeviceToHost));
+    for (int64_t i = 0; i < nnz; ++i) ent_idx[i] += 1;
+  }
+  if (val && nnz) NN_CUDA(cudaMemcpy(val, h->d_val.as<double>() + s0, (size_t)nnz * 8, cudaMemcpyDeviceToHost));
   return NNSDP_OK;
 }
 

@@ -380,15 +380,30 @@ struct AffineDev {
   long long nvar, var_out, var_bnd, var_sec;  // variable layout: [gin | gout | gbnd | gsec]
   long long acdim, lamdim, beta;
   int out_kind;
-  const double *x1min, *x1max, *ymin, *ymax, *smin, *smax;  // one query
+  const double *x1min, *x1max, *ymin, *ymax, *smin, *smax;  // one query (the batched form: query 0)
+  long long s_x1min, s_x1max, s_ymin, s_ymax, s_smin, s_smax;  // batched form: strides between queries
   const long long* col_ptr;  // Zdim + 1 : first cover entry of every column (upper triangle, column-major)
   const int* lo;             // Zdim     : first row of column c inside the cover
 };
 int launch_affine_count(const NetDev& net, const AffineDev& A, long long* counts, cudaStream_t st);
 int launch_affine_fill(const NetDev& net, const AffineDev& A, const long long* offs, long long* ent,
                        long long* var, double* val, cudaStream_t st);
-int launch_affine_z0(const NetDev& net, const BatchDev& b, const AffineDev& A, double* z0,
+// z0[q * nent + e] for the Q queries of the batch (all multipliers zero)
+int launch_affine_z0(const NetDev& net, const BatchDev& b, const AffineDev& A, long long nent, int Q, double* z0,
                      cudaStream_t st);
+// Batched form: canonical CSC of every group (the bounds of group g are those of query first[g]).
+// counts[g * nvar + v] = merged coefficients of variable v in group g; after an exclusive scan over (group, variable)
+// the fill writes variable v of group g at offs[g * nvar + v], entries (0-based) ascending.
+int launch_affine_csc_count(const NetDev& net, const AffineDev& A, const long long* first, long long ngroups,
+                            long long* counts, cudaStream_t st);
+int launch_affine_csc_fill(const NetDev& net, const AffineDev& A, const long long* first, long long ngroups,
+                           const long long* offs, long long* ent, double* val, cudaStream_t st);
+// exclusive scan of x[0..n) in place; sums = scratch of scan_scratch_len(n) elements
+long long scan_scratch_len(long long n);
+int launch_scan_exclusive(long long* x, long long n, long long* sums, cudaStream_t st);
+// starts[g] = offs[g * nvar], g = 0..ngroups
+int launch_affine_group_starts(const long long* offs, long long nvar, long long ngroups, long long* starts,
+                               cudaStream_t st);
 
 // matrix-free lambda_max (kernels_eig.cu); Qc = queries of the current chunk, first one is q_first
 int launch_eig_init(double* v, int Zdim, int Qc, int q_first, cudaStream_t st);

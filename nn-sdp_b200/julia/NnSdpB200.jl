@@ -360,8 +360,80 @@ function affineForm(net::DeviceNet, β::Int, qc_input, qc_out, qc_bounded, qc_se
   return s, ent_row, ent_col, z0, A
 end
 
+# The affine forms of several queries in one call (nnsdp_affine_create_batch): the directions of a reach polytope
+# (src/NnSdp.jl:73-95) or the members of a vnnlib property (experiments/vnnlib_utils.jl:58-74).  The queries share one
+# output-QC type; their boxes, QC bounds and output data are packed as Q-column arrays.  Queries with the same box and
+# QC bounds share one coefficient matrix, built once on the device as canonical CSC (no sort, no duplicate sum here):
+# `A` is then the same SparseMatrixCSC object for every member of the group.  Returns one
+# (sizes, ent_row, ent_col, z0, A) per query, as affineForm does for one.
+struct AffineBatchSizes
+  Q::Int64; ngroups::Int64
+  nvar::Int64; nent::Int64
+  var_in::Int64; var_out::Int64; var_bnd::Int64; var_sec::Int64
+  nnz_total::Int64; nnz_max::Int64
+end
+
+function affineFormBatch(net::DeviceNet, β::Int, queries; max_nnz::Int = 0)
+  Q = length(queries)
+  Q >= 1 || error("affineFormBatch needs at least one query")
+  outs = [q isa Methods.SafetyQuery ? q.qc_safety : q.qc_reach for q in queries]
+  all(o -> typeof(o) == typeof(outs[1]), outs) || error("affineFormBatch: the queries must share one output-QC type")
+  cols(f) = reduce(hcat, [Vector{Float64}(f(i)) for i in 1:Q])   # n x Q: column q belongs to query q
+  x1min, x1max = cols(i -> queries[i].qc_input.x1min), cols(i -> queries[i].qc_input.x1max)
+  ymin, ymax = cols(i -> queries[i].qc_activs[1].acymin), cols(i -> queries[i].qc_activs[1].acymax)
+  smin, smax = cols(i -> queries[i].qc_activs[2].smin), cols(i -> queries[i].qc_activs[2].smax)
+  kind, S, vec, invP = OUT_SAFETY, zeros(0, 0), zeros(0, 0), zeros(0, 0)
+  o1 = outs[1]
+  if o1 isa QcSafety
+    S = cols(i -> vec_colmajor(Matrix{Float64}(outs[i].S)))
+  elseif o1 isa QcReachHplane
+    kind, vec = OUT_HPLANE, cols(i -> outs[i].normal)
+  elseif o1 isa QcReachCircle
+    kind, vec = OUT_CIRCLE, cols(i -> outs[i].yc)
+  elseif o1 isa QcReachEllipsoid
+    kind, vec = OUT_ELLIPSOID, cols(i -> outs[i].yc)
+    invP = cols(i -> vec_colmajor(Matrix{Float64}(outs[i].invP)))
+  else
+    error("unrecognized qc: $(o1)")   # src/Qc/output.jl:95
+  end
+  zin, zbnd, zsec, zout = zeros(size(x1min, 1)), zeros(size(ymin, 1)), zeros(queries[1].qc_activs[2].vardim), [0.0]
+  p(a) = isempty(a) ? Ptr{Float64}(C_NULL) : pointer(a)
+  ld(a) = Int64(size(a, 1))
+  keep = Any[x1min, x1max, ymin, ymax, smin, smax, S, vec, invP, zin, zbnd, zsec, zout]
+  qi = Ref(QueryInputs(p(x1min), ld(x1min), p(x1max), ld(x1max), p(ymin), ld(ymin), p(ymax), ld(ymax),
+                       p(smin), ld(smin), p(smax), ld(smax), p(zin), 0, p(zbnd), 0, p(zsec), 0, kind, Int32(0),
+                       p(S), ld(S), p(vec), ld(vec), p(invP), ld(invP),
+                       kind == OUT_SAFETY ? Ptr{Float64}(C_NULL) : p(zout), 0))
+  h, sz = Ref{Ptr{Cvoid}}(C_NULL), Ref{AffineBatchSizes}()
+  GC.@preserve keep check(ccall((:nnsdp_affine_create_batch, LIB), Int32,
+      (Ptr{Cvoid}, Ptr{Cvoid}, Int64, Int64, Ptr{QueryInputs}, Int64, Ptr{Ptr{Cvoid}}, Ptr{AffineBatchSizes}),
+      net.ctx.h, net.h, β, Q, qi, max_nnz, h, sz))
+  s = sz[]
+  ent_row, ent_col, z0 = zeros(Int64, s.nent), zeros(Int64, s.nent), zeros(s.nent, Q)
+  group_of, group_nnz, group_first = zeros(Int64, Q), zeros(Int64, s.ngroups), zeros(Int64, s.ngroups)
+  mats = Vector{SparseMatrixCSC{Float64, Int64}}(undef, s.ngroups)
+  try
+    check(ccall((:nnsdp_affine_batch_get, LIB), Int32, (Ptr{Cvoid}, Ptr{Int64}, Ptr{Int64}, Ptr{Float64}),
+                h[], ent_row, ent_col, z0))
+    check(ccall((:nnsdp_affine_batch_groups, LIB), Int32, (Ptr{Cvoid}, Ptr{Int64}, Ptr{Int64}, Ptr{Int64}),
+                h[], group_of, group_nnz, group_first))
+    for g in 1:s.ngroups
+      var_ptr, ent_idx, val = zeros(Int64, s.nvar + 1), zeros(Int64, group_nnz[g]), zeros(group_nnz[g])
+      check(ccall((:nnsdp_affine_batch_get_group, LIB), Int32, (Ptr{Cvoid}, Int64, Ptr{Int64}, Ptr{Int64}, Ptr{Float64}),
+                  h[], g - 1, var_ptr, ent_idx, val))
+      mats[g] = SparseMatrixCSC(s.nent, s.nvar, var_ptr, ent_idx, val)   # canonical: no sort, no duplicate sum
+    end
+  finally
+    ccall((:nnsdp_affine_batch_destroy, LIB), Int32, (Ptr{Cvoid},), h[])
+  end
+  sizes_of(A) = AffineSizes(s.nvar, s.nent, nnz(A), s.var_in, s.var_out, s.var_bnd, s.var_sec)
+  return [(sizes_of(mats[group_of[q] + 1]), ent_row, ent_col, z0[:, q], mats[group_of[q] + 1]) for q in 1:Q]
+end
+
 # Options type that selects the GPU-assembled constraints in runQuery (src/Methods/Methods.jl:97-103);
 # same five fields as ChordalSdpOptions (src/Methods/chordal_sdp.jl:10-16) plus the device network.
+# `forms`: query => affineForm result, e.g. from affineFormBatch for a polytope or a vnnlib property; setupB200! then
+# uses that entry instead of calling affineForm.
 Base.@kwdef struct ChordalB200Options <: Methods.QueryOptions
   include_default_mosek_opts::Bool = true
   mosek_opts::Dict{String, Any} = Dict()
@@ -369,6 +441,7 @@ Base.@kwdef struct ChordalB200Options <: Methods.QueryOptions
   use_dual::Bool = false
   verbose::Bool = false
   net::DeviceNet
+  forms::Union{Nothing, IdDict} = nothing
 end
 
 # Common part of setupSafety!/setupReach! (src/Methods/chordal_sdp.jl:96-153): variables in the reference's
@@ -379,7 +452,8 @@ function setupB200!(model, query, qc_out, opts::ChordalB200Options)
   ffnet = query.ffnet
   qc_bounded, qc_sector = query.qc_activs[1], query.qc_activs[2]   # order of makeQcActivsIntvs (activ.jl:64)
   β = qc_sector.β
-  s, ent_row, ent_col, z0, A = affineForm(opts.net, β, query.qc_input, qc_out, qc_bounded, qc_sector)
+  s, ent_row, ent_col, z0, A = (opts.forms !== nothing && haskey(opts.forms, query)) ? opts.forms[query] :
+                                affineForm(opts.net, β, query.qc_input, qc_out, qc_bounded, qc_sector)
   vars = Dict()
   γin = Methods.JuMP.@variable(model, [1:query.qc_input.vardim])
   Methods.JuMP.@constraint(model, γin .>= 0)
@@ -433,6 +507,6 @@ function Methods.setupReach!(model, query::Methods.ReachQuery, opts::ChordalB200
 end
 
 export Context, DeviceNet, IntervalsB200, IntervalsCrownB200, makeCliquesB200, assembleCliqueBlocks, assembleZ
-export affineForm, ChordalB200Options, eigmaxZ, packedLayout, cellView, assemblePacked, cliqueBlocks
+export affineForm, affineFormBatch, ChordalB200Options, eigmaxZ, packedLayout, cellView, assemblePacked, cliqueBlocks
 
 end # module

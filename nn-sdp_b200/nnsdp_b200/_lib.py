@@ -39,6 +39,14 @@ class AffineSizes(C.Structure):
         return {n: int(getattr(self, n)) for n, _ in self._fields_}
 
 
+class AffineBatchSizes(C.Structure):
+    _fields_ = [(n, c_i64) for n in ("Q", "ngroups", "nvar", "nent", "var_in", "var_out", "var_bnd", "var_sec",
+                                     "nnz_total", "nnz_max")]
+
+    def as_dict(self):
+        return {n: int(getattr(self, n)) for n, _ in self._fields_}
+
+
 class PackedCell(C.Structure):
     _fields_ = [("kind", C.c_int32), ("blk", C.c_int32), ("row0", C.c_int64), ("col0", C.c_int64), ("nrows", C.c_int64),
                 ("ncols", C.c_int64), ("offset", C.c_int64), ("always", C.c_int32), ("reserved", C.c_int32)]
@@ -98,6 +106,12 @@ PROTOTYPES = {
     "nnsdp_affine_create": (c_i32, [c_vp, c_vp, c_i64, C.POINTER(QueryInputs), c_i64, C.POINTER(c_vp), C.POINTER(AffineSizes)]),
     "nnsdp_affine_get": (c_i32, [c_vp, c_i64p, c_i64p, c_dp, c_i64p, c_i64p, c_dp]),
     "nnsdp_affine_destroy": (c_i32, [c_vp]),
+    "nnsdp_affine_create_batch": (c_i32, [c_vp, c_vp, c_i64, c_i64, C.POINTER(QueryInputs), c_i64, C.POINTER(c_vp),
+                                          C.POINTER(AffineBatchSizes)]),
+    "nnsdp_affine_batch_groups": (c_i32, [c_vp, c_i64p, c_i64p, c_i64p]),
+    "nnsdp_affine_batch_get": (c_i32, [c_vp, c_i64p, c_i64p, c_dp]),
+    "nnsdp_affine_batch_get_group": (c_i32, [c_vp, c_i64, c_i64p, c_i64p, c_dp]),
+    "nnsdp_affine_batch_destroy": (c_i32, [c_vp]),
     "nnsdp_batch_create": (c_i32, [c_vp, c_i32, c_vp, c_i64, c_i64, c_i64, c_i32, C.POINTER(c_vp)]),
     "nnsdp_batch_destroy": (c_i32, [c_vp]),
     "nnsdp_batch_set_inputs": (c_i32, [c_vp, c_i64, C.POINTER(QueryInputs)]),

@@ -421,6 +421,37 @@ def affine_form(net: Net, beta: int, batch: NumericBatch, max_nnz: int = 0) -> d
         L.lib.nnsdp_affine_destroy(h)
 
 
+def affine_form_batch(net: Net, beta: int, batch: NumericBatch, Q: Optional[int] = None, max_nnz: int = 0) -> dict:
+    """The affine forms of Q queries in one call (nnsdp_affine_create_batch).  Queries with the same box (and the same
+    bounds, when the batch carries them) share one coefficient matrix.  Returns the sizes, the 1-based entry positions,
+    z0 of shape (Q, nent), group_of (0-based) and `groups`: per group a dict with the canonical CSC arrays of its
+    nent x nvar matrix (`var_ptr`, `ent_idx`, both 1-based, and `val`) and `first`, its first query."""
+    Q = Q or _infer_Q(batch)
+    qi, keep = batch.pack(Q)
+    h, sz = L.c_vp(), L.AffineBatchSizes()
+    L.check(L.lib.nnsdp_affine_create_batch(net.ctx._h, net._h, beta, Q, C.byref(qi), max_nnz, C.byref(h),
+                                            C.byref(sz)))
+    try:
+        d = sz.as_dict()
+        G, ip = d["ngroups"], (lambda a: a.ctypes.data_as(L.c_i64p))
+        out = {"ent_row": np.zeros(d["nent"], dtype=np.int64), "ent_col": np.zeros(d["nent"], dtype=np.int64),
+               "z0": np.zeros((Q, d["nent"])), "group_of": np.zeros(Q, dtype=np.int64)}
+        nnz, first = np.zeros(G, dtype=np.int64), np.zeros(G, dtype=np.int64)
+        L.check(L.lib.nnsdp_affine_batch_get(h, ip(out["ent_row"]), ip(out["ent_col"]), _dp(out["z0"])))
+        L.check(L.lib.nnsdp_affine_batch_groups(h, ip(out["group_of"]), ip(nnz), ip(first)))
+        groups = []
+        for g in range(G):
+            grp = {"var_ptr": np.zeros(d["nvar"] + 1, dtype=np.int64), "ent_idx": np.zeros(nnz[g], dtype=np.int64),
+                   "val": np.zeros(nnz[g]), "first": int(first[g])}
+            L.check(L.lib.nnsdp_affine_batch_get_group(h, g, ip(grp["var_ptr"]), ip(grp["ent_idx"]), _dp(grp["val"])))
+            groups.append(grp)
+        out["groups"] = groups
+        out.update(d)
+        return out
+    finally:
+        L.lib.nnsdp_affine_batch_destroy(h)
+
+
 def split_blocks(flat: np.ndarray, cliques) -> List[np.ndarray]:
     """One query's flat output -> list of |Ck| x |Ck| matrices ([r, c] indexing)."""
     out, o = [], 0
