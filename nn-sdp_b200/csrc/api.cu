@@ -897,17 +897,22 @@ int32_t nnsdp_batch_create(nnsdp_ctx* ctx, int32_t dev_index, const nnsdp_net* n
     b->pd.mats = b->d_mats.as<MatDev>();
     b->pd.panel_desc = nullptr;
     b->pd.n_panel = 0;
+    b->pd.fold = 0;
     {
-      // dense formats of wide nets: fill strips and window tiles in one launch in panel order (plan.cpp build_panel,
-      // emit_panel_kernel).  NNSDP_PANEL=0 keeps the two kernels.
+      // dense formats of wide nets: fill strips, window tiles and edge tiles in one launch in panel order (plan.cpp,
+      // emit_panel_kernel), then the bulk strips of the pass and the band.  NNSDP_PANEL=0 keeps the separate fill and
+      // window kernels; NNSDP_PANEL_FOLD=0 (read per batch) keeps the edge tiles in a launch of their own.
       static const int panel_env = [] { const char* e = getenv("NNSDP_PANEL"); return e ? atoi(e) : 1; }();
       if (panel_env && !b->packed && !b->plan.panel.empty()) {
+        const char* fold_env = getenv("NNSDP_PANEL_FOLD");
+        const bool fold = !(fold_env && atoi(fold_env) == 0);
         std::vector<StripDev> panel;
-        for (const StripDev& d : b->plan.panel)
+        for (const StripDev& d : fold ? b->plan.panel_fold : b->plan.panel)
           if (d.prog != PROG_ZERO && (d.prog == PROG_RC || d.prog == PROG_CR || !is_bulk(d))) panel.push_back(d);
         NN_TRY(upload(b->d_panel, panel.data(), panel.size() * sizeof(StripDev), b->st));
         b->pd.panel_desc = b->d_panel.as<StripDev>();
         b->pd.n_panel = (int)panel.size();
+        b->pd.fold = fold ? 1 : 0;
       }
     }
     b->pd.ntiles = (int)b->plan.tiles.size();
@@ -1221,7 +1226,8 @@ static int32_t prepare_slots(nnsdp_batch* b, int64_t q0, int64_t nq, int64_t p0)
   return NNSDP_OK;
 }
 
-// One emitter pass = fill, window and edge kernels back to back, each inside its own CUDA-event span
+// One emitter pass = fill, window and edge kernels back to back (with PlanDev::fold the edge tiles are part of the
+// panel launch), each inside its own CUDA-event span
 // (ST_EMIT_FILL / _WINDOW / _EDGE) so that the per-kernel launch durations can be read back.
 static int32_t emit_pass(nnsdp_batch* b, const GramDev& gd, int q0, int nq, double* dst) {
   const NetPerDev& nd = *b->nd;

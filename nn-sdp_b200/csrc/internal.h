@@ -190,6 +190,9 @@ struct PlanHost {
   // window tiles re-packed into the strip layout (prog = PROG_RC / PROG_CR, rl0 = cblk, cl0 = flags, ldG = matrix order).
   // Empty when the plan keeps the two kernels.
   std::vector<StripDev> panel;
+  // The same list with the edge tiles (MIXED / GENERAL, re-packed like the window tiles) sorted in; empty exactly when
+  // `panel` is.
+  std::vector<StripDev> panel_fold;
 };
 
 // ---------------------------------------------------------------------------------
@@ -304,6 +307,7 @@ struct PlanDev {
   const StripDev* panel_desc;  // n_panel work items of the panel-ordered launch: AFF strips as they are; window tiles re-packed
                              // (prog = PROG_RC / PROG_CR, rblk, rl0 = cblk, cl0 = flags, ldG = matrix order)
   int n_panel;               // 0: fill and window kernels run one after the other
+  int fold;                  // panel_desc also holds the edge tiles (PlanHost::panel_fold): no edge launch
   int ntiles;                // tiles are sorted: [fill | window | edge]
   int n_fill, n_window, n_edge;
   int tile_rows;

@@ -611,69 +611,13 @@ emit_window_kernel(NetDev net, BatchDev b, PlanDev plan, int tile0, int q0, int 
   }
 }
 
-// ---- kernels 1 + 2 as one launch in PANEL order (dense formats of wide nets) ----------------------------------
-// A column of a clique block is written by several programs: fill strips (affine pieces; the Gram pieces go out in
-// their own launch, for the (slot, block) pairs that need them) and window tiles.  Launched one kernel after the
-// other, the pieces of a column reach DRAM milliseconds apart and each launch covers only part of every DRAM page it
-// touches (tools/probe_write_bw.cu: two launches 5.7 TB/s, one launch with the items ordered by 32-column panel
-// 7.0 TB/s on pure stores).  Here the work items of both kernels are sorted by
-// (matrix, 32-column panel, row) and consecutive CTAs take consecutive items, so whole columns are written within
-// microseconds.  Inside a sub-batch of queries (see below) a window CTA writes its tile for `group` consecutive queries and
-// a strip CTA its strip for every (batch / group)-th query.
-template <int BETA>
-__global__ void __launch_bounds__(ETHREADS, 4)
-emit_panel_kernel(NetDev net, BatchDev b, GramDev g, PlanDev plan, int q0, int nq, int group, double* __restrict__ out) {
-  constexpr int RC_DOUBLES = SLOT_GROUP * (BETA + 1) * (FAST_TC + BETA + 1), CR_DOUBLES = FAST_TC * CR_LDW(BETA);
-  __shared__ __align__(128) double smem[RC_DOUBLES > CR_DOUBLES ? RC_DOUBLES : CR_DOUBLES];
-  __shared__ __align__(8) unsigned long long mbar;
-  // CTA order: the queries of a pass go in sub-batches of `batch` (a multiple of group): all items for the first
-  // sub-batch, then all items for the next one.  Fewer queries in flight at a time = fewer DRAM pages open at a time:
-  // a 16-query pass runs at 5.75 TB/s and an 8-query pass at 5.83 TB/s where a 32-query pass reaches 5.58 TB/s.
-  const int batch = group >> 8;
-  group &= 255;
-  const int gb = batch / group;                         // CTAs per item and full sub-batch
-  const int per_batch = plan.n_panel * gb;
-  const int sb = blockIdx.x / per_batch, rem = blockIdx.x - sb * per_batch;
-  const int slot_lo = sb * batch, slot_hi = min(nq, slot_lo + batch);
-  const int item = rem / gb, g0 = rem - item * gb;
-  // one self-contained 64 B descriptor per item, in panel order: a fill strip as it is, a window tile re-packed into
-  // the same layout (no index -> tile -> matrix chain of dependent loads at the start of a short CTA)
-  const StripDev* desc = plan.panel_desc + item;
-  const int4* dp = reinterpret_cast<const int4*>(desc);
-  const int4 d2 = __ldg(dp + 2);
-  if (d2.w != PROG_RC && d2.w != PROG_CR) {
-    for (int slot = slot_lo + g0; slot < slot_hi; slot += gb) fill_strip<false>(net, b, g, plan, desc, slot, q0, out);
-    return;
-  }
-  const int4 d0 = __ldg(dp), d1 = __ldg(dp + 1), d3 = __ldg(dp + 3);
-  TileDev t;
-  t.mat = 0;
-  t.row0 = d1.y, t.nrows = d1.z, t.col0 = d1.w, t.ncols = d2.x, t.grow0 = d2.y, t.gcol0 = d2.z, t.prog = d2.w;
-  t.rblk = d3.x, t.cblk = d3.y, t.flags = (uint32_t)d3.z;
-  MatDev mat;
-  mat.out_off = ((long long)(unsigned)d0.x) | ((long long)d0.y << 32);
-  mat.ld = d1.x;
-  mat.n = d3.w;
-  const int slot0 = slot_lo + g0 * group;
-  const int nslots = min(group, slot_hi - slot0);
-  if (nslots <= 0) return;
-  if (t.prog == PROG_RC) {
-    if (t.ncols == FAST_TC) emit_rc<BETA, true>(net, b, plan, t, mat, q0, slot0, nslots, out, smem);
-    else emit_rc<BETA, false>(net, b, plan, t, mat, q0, slot0, nslots, out, smem);
-  } else {
-    emit_cr<BETA>(net, b, plan, t, mat, q0, slot0, nslots, out, smem, &mbar);
-  }
-}
-
 // ---- kernel 3: everything else (band / sliver / corner tiles, affine row and column, small nets) -
-__global__ void __launch_bounds__(ETHREADS, 4)
-emit_edge_kernel(NetDev net, BatchDev b, GramDev g, PlanDev plan, int tile0, int q0, int nq,
-                 int group, double* __restrict__ out) {
-  __shared__ double smem[MAX_TC * MAX_TAPS + 128 * MAX_TAPS];
-  const TileDev t = plan.tiles[tile0 + blockIdx.x];
-  const MatDev mat = plan.mats[t.mat];
-  const int slot0 = blockIdx.y * group;
-  const int nslots = min(group, nq - slot0);
+constexpr int EDGE_DOUBLES = MAX_TC * MAX_TAPS + 128 * MAX_TAPS;  // shared memory of emit_mixed
+
+// One MIXED / GENERAL tile for the queries (ring slots) [slot0, slot0 + nslots)
+__device__ __forceinline__ void emit_edge_tile(const NetDev& net, const BatchDev& b, const GramDev& g,
+                                               const PlanDev& plan, const TileDev& t, const MatDev& mat, int q0,
+                                               int slot0, int nslots, double* __restrict__ out, double* smem) {
   // thread = (row, column group); thin sliver tiles (2 x 32, 128 x 2, ...) spread their few entries over
   // as many threads as possible: rows per column group = smallest power of two covering the tile's rows
   int TR = 1;
@@ -702,6 +646,80 @@ emit_edge_kernel(NetDev net, BatchDev b, GramDev g, PlanDev plan, int tile0, int
     const QView v = make_view(net, b, g, q0 + slot0 + s, slot0 + s);
     double* o = out + (long long)(slot0 + s) * plan.per_query + tile_off;
     emit_general(net, b, g, t, mat, v, o, tr, cg2, TC);
+  }
+}
+
+__global__ void __launch_bounds__(ETHREADS, 4)
+emit_edge_kernel(NetDev net, BatchDev b, GramDev g, PlanDev plan, int tile0, int q0, int nq,
+                 int group, double* __restrict__ out) {
+  __shared__ double smem[EDGE_DOUBLES];
+  const TileDev t = plan.tiles[tile0 + blockIdx.x];
+  const MatDev mat = plan.mats[t.mat];
+  const int slot0 = blockIdx.y * group;
+  emit_edge_tile(net, b, g, plan, t, mat, q0, slot0, min(group, nq - slot0), out, smem);
+}
+
+// ---- kernels 1 + 2 (+ 3) as one launch in PANEL order (dense formats of wide nets) -----------------------------
+// A column of a clique block is written by several programs: fill strips (affine pieces; the Gram pieces go out in
+// their own launch, for the (slot, block) pairs that need them), window tiles and edge tiles (slivers, corners).  Launched one kernel after the
+// other, the pieces of a column reach DRAM milliseconds apart and each launch covers only part of every DRAM page it
+// touches (tools/probe_write_bw.cu: two launches 5.7 TB/s, one launch with the items ordered by 32-column panel
+// 7.0 TB/s on pure stores).  Here the work items of both kernels are sorted by
+// (matrix, 32-column panel, row) and consecutive CTAs take consecutive items, so whole columns are written within
+// microseconds.  Inside a sub-batch of queries (see below) a window CTA writes its tile for `group` consecutive queries and
+// a strip CTA its strip for every (batch / group)-th query.  FOLD: the list holds the edge tiles too, and the first CTA
+// of an edge item writes its tile for every query of the sub-batch (the others have nothing to do): a stress pass takes
+// 2.90 ms this way, 2.94 ms with the queries spread over the item's CTAs like a strip's, 3.00 ms with the separate edge
+// launch (one B200).  Both forms store the same bits.
+template <int BETA, bool FOLD>
+__global__ void __launch_bounds__(ETHREADS, 4)
+emit_panel_kernel(NetDev net, BatchDev b, GramDev g, PlanDev plan, int q0, int nq, int group, double* __restrict__ out) {
+  constexpr int RC_DOUBLES = SLOT_GROUP * (BETA + 1) * (FAST_TC + BETA + 1), CR_DOUBLES = FAST_TC * CR_LDW(BETA);
+  constexpr int WIN_DOUBLES = RC_DOUBLES > CR_DOUBLES ? RC_DOUBLES : CR_DOUBLES;
+  static_assert(WIN_DOUBLES >= EDGE_DOUBLES, "the edge tiles stage their band coefficients in the same buffer");
+  __shared__ __align__(128) double smem[WIN_DOUBLES];
+  __shared__ __align__(8) unsigned long long mbar;
+  // CTA order: the queries of a pass go in sub-batches of `batch` (a multiple of group): all items for the first
+  // sub-batch, then all items for the next one.  Fewer queries in flight at a time = fewer DRAM pages open at a time:
+  // a 16-query pass runs at 5.75 TB/s and an 8-query pass at 5.83 TB/s where a 32-query pass reaches 5.58 TB/s.
+  const int batch = group >> 8;
+  group &= 255;
+  const int gb = batch / group;                         // CTAs per item and full sub-batch
+  const int per_batch = plan.n_panel * gb;
+  const int sb = blockIdx.x / per_batch, rem = blockIdx.x - sb * per_batch;
+  const int slot_lo = sb * batch, slot_hi = min(nq, slot_lo + batch);
+  const int item = rem / gb, g0 = rem - item * gb;
+  // one self-contained 64 B descriptor per item, in panel order: a fill strip as it is, a window tile re-packed into
+  // the same layout (no index -> tile -> matrix chain of dependent loads at the start of a short CTA)
+  const StripDev* desc = plan.panel_desc + item;
+  const int4* dp = reinterpret_cast<const int4*>(desc);
+  const int4 d2 = __ldg(dp + 2);
+  if (d2.w != PROG_RC && d2.w != PROG_CR && !(FOLD && (d2.w == PROG_MIXED || d2.w == PROG_GENERAL))) {
+    for (int slot = slot_lo + g0; slot < slot_hi; slot += gb) fill_strip<false>(net, b, g, plan, desc, slot, q0, out);
+    return;
+  }
+  if (FOLD && (d2.w == PROG_MIXED || d2.w == PROG_GENERAL) && g0 != 0) return;
+  const int4 d0 = __ldg(dp), d1 = __ldg(dp + 1), d3 = __ldg(dp + 3);
+  TileDev t;
+  t.mat = 0;
+  t.row0 = d1.y, t.nrows = d1.z, t.col0 = d1.w, t.ncols = d2.x, t.grow0 = d2.y, t.gcol0 = d2.z, t.prog = d2.w;
+  t.rblk = d3.x, t.cblk = d3.y, t.flags = (uint32_t)d3.z;
+  MatDev mat;
+  mat.out_off = ((long long)(unsigned)d0.x) | ((long long)d0.y << 32);
+  mat.ld = d1.x;
+  mat.n = d3.w;
+  if (FOLD && t.prog != PROG_RC && t.prog != PROG_CR) {
+    emit_edge_tile(net, b, g, plan, t, mat, q0, slot_lo, slot_hi - slot_lo, out, smem);
+    return;
+  }
+  const int slot0 = slot_lo + g0 * group;
+  const int nslots = min(group, slot_hi - slot0);
+  if (nslots <= 0) return;
+  if (t.prog == PROG_RC) {
+    if (t.ncols == FAST_TC) emit_rc<BETA, true>(net, b, plan, t, mat, q0, slot0, nslots, out, smem);
+    else emit_rc<BETA, false>(net, b, plan, t, mat, q0, slot0, nslots, out, smem);
+  } else {
+    emit_cr<BETA>(net, b, plan, t, mat, q0, slot0, nslots, out, smem, &mbar);
   }
 }
 
@@ -822,13 +840,18 @@ int launch_emit(const NetDev& net, const BatchDev& b, const GramDev& g, const Pl
       if (pbatch > 255) pbatch = (255 / pgroup) * pgroup;
       const int nbatches = (nq + pbatch - 1) / pbatch;
       const dim3 grid((unsigned)plan.n_panel * (pbatch / pgroup) * nbatches);
+      const int gp = pgroup | (pbatch << 8);
+#define NNSDP_PANEL_LAUNCH(B)                                                                                  \
+  if (plan.fold) emit_panel_kernel<B, true><<<grid, ETHREADS, 0, st>>>(net, b, g, plan, q0, nq, gp, out);      \
+  else emit_panel_kernel<B, false><<<grid, ETHREADS, 0, st>>>(net, b, g, plan, q0, nq, gp, out);
       switch (b.beta) {
-        case 0: emit_panel_kernel<0><<<grid, ETHREADS, 0, st>>>(net, b, g, plan, q0, nq, pgroup | (pbatch << 8), out); break;
-        case 1: emit_panel_kernel<1><<<grid, ETHREADS, 0, st>>>(net, b, g, plan, q0, nq, pgroup | (pbatch << 8), out); break;
-        case 2: emit_panel_kernel<2><<<grid, ETHREADS, 0, st>>>(net, b, g, plan, q0, nq, pgroup | (pbatch << 8), out); break;
-        case 3: emit_panel_kernel<3><<<grid, ETHREADS, 0, st>>>(net, b, g, plan, q0, nq, pgroup | (pbatch << 8), out); break;
-        default: emit_panel_kernel<4><<<grid, ETHREADS, 0, st>>>(net, b, g, plan, q0, nq, pgroup | (pbatch << 8), out); break;
+        case 0: NNSDP_PANEL_LAUNCH(0) break;
+        case 1: NNSDP_PANEL_LAUNCH(1) break;
+        case 2: NNSDP_PANEL_LAUNCH(2) break;
+        case 3: NNSDP_PANEL_LAUNCH(3) break;
+        default: NNSDP_PANEL_LAUNCH(4) break;
       }
+#undef NNSDP_PANEL_LAUNCH
       ++launches;
     }
   } else {
@@ -857,7 +880,7 @@ int launch_emit(const NetDev& net, const BatchDev& b, const GramDev& g, const Pl
   }
   }
   if (which < 0 || which == 0) launches += launch_bulk(net, b, g, plan, q0, sel, nsel, out, st);
-  if (plan.n_edge > 0 && (which < 0 || which == 2)) {
+  if (!plan.fold && plan.n_edge > 0 && (which < 0 || which == 2)) {
     emit_edge_kernel<<<dim3(plan.n_edge, (nq + egroup - 1) / egroup), ETHREADS, 0, st>>>(
         net, b, g, plan, plan.n_fill + plan.n_window, q0, nq, egroup, out);
     ++launches;

@@ -639,32 +639,22 @@ int32_t build_plan(const Shape& sh, int64_t beta, const std::vector<CliqueRanges
   // consecutive CTAs of one launch.  Dense formats of wide nets only: packed cells are contiguous per program, and
   // narrow layers are issue-bound, not locality-bound (profiles/r2_experiments.txt).
   plan->panel.clear();
+  plan->panel_fold.clear();
   if (!packed && !plan->band_inline && plan->n_window > 0 && beta <= MAX_WINDOW_BETA) {
-    struct Key { long long off; int panel, row0, col0, code; };
+    struct Key { long long off; int panel, row0, col0; StripDev d; };
     std::vector<Key> keys;
-    keys.reserve((size_t)plan->n_fill + plan->n_window);
-    for (int i = 0; i < plan->n_fill; ++i) {
-      const StripDev& d = plan->strips[i];
-      keys.push_back({d.out_off, d.col0 / 32, d.row0, d.col0, i});
-    }
-    for (int i = 0; i < plan->n_window; ++i) {
-      const TileDev& t = plan->tiles[plan->n_fill + i];
-      keys.push_back({plan->mats[t.mat].out_off, t.col0 / 32, t.row0, t.col0, ~i});
-    }
-    std::stable_sort(keys.begin(), keys.end(), [](const Key& x, const Key& y) {
-      if (x.off != y.off) return x.off < y.off;
-      if (x.panel != y.panel) return x.panel < y.panel;
-      if (x.col0 != y.col0) return x.col0 < y.col0;
-      return x.row0 < y.row0;
-    });
-    plan->panel.resize(keys.size());
-    for (size_t i = 0; i < keys.size(); ++i) {
-      const int code = keys[i].code;
-      if (code >= 0) {
-        plan->panel[i] = plan->strips[code];
-        continue;
-      }
-      const TileDev& t = plan->tiles[plan->n_fill + ~code];
+    auto sorted = [](std::vector<Key> k) {
+      std::stable_sort(k.begin(), k.end(), [](const Key& x, const Key& y) {
+        if (x.off != y.off) return x.off < y.off;
+        if (x.panel != y.panel) return x.panel < y.panel;
+        if (x.col0 != y.col0) return x.col0 < y.col0;
+        return x.row0 < y.row0;
+      });
+      std::vector<StripDev> v(k.size());
+      for (size_t i = 0; i < k.size(); ++i) v[i] = k[i].d;
+      return v;
+    };
+    auto add_tile = [&](const TileDev& t) {  // window / edge tile re-packed into the strip layout
       const MatDev& m = plan->mats[t.mat];
       StripDev d{};
       d.out_off = m.out_off;
@@ -672,8 +662,16 @@ int32_t build_plan(const Shape& sh, int64_t beta, const std::vector<CliqueRanges
       d.row0 = t.row0; d.nrows = t.nrows; d.col0 = t.col0; d.ncols = t.ncols;
       d.grow0 = t.grow0; d.gcol0 = t.gcol0; d.prog = t.prog;
       d.rblk = t.rblk; d.rl0 = t.cblk; d.cl0 = (int32_t)t.flags; d.ldG = m.n;
-      plan->panel[i] = d;
+      keys.push_back({d.out_off, d.col0 / 32, d.row0, d.col0, d});
+    };
+    for (int i = 0; i < plan->n_fill; ++i) {
+      const StripDev& d = plan->strips[i];
+      keys.push_back({d.out_off, d.col0 / 32, d.row0, d.col0, d});
     }
+    for (int i = 0; i < plan->n_window; ++i) add_tile(plan->tiles[plan->n_fill + i]);
+    plan->panel = sorted(keys);
+    for (int i = 0; i < plan->n_edge; ++i) add_tile(plan->tiles[plan->n_fill + plan->n_window + i]);
+    plan->panel_fold = sorted(keys);
   }
   return NNSDP_OK;
 }
