@@ -380,6 +380,34 @@ int32_t nnsdp_batch_lambda_max_ex(nnsdp_batch* batch, int32_t max_iters, double 
 int32_t nnsdp_batch_lambda_max(nnsdp_batch* batch, int32_t max_iters, double tol, double* lam_max,
                                int32_t* iters);
 
+/* ---- sound certificate eigmax(Z) <= tau (DESIGN.md section 9) --------------------------------------------------
+ * For every query of a prepared batch in NNSDP_FORMAT_BLOCKS with ring_queries > 0: emits the query's clique blocks
+ * into a ring slot and factorises tau' I - Z in place, clique by clique (multifrontal Cholesky along the path of
+ * cliques, natural elimination order; the FP64 tensor cores do the trailing updates).  tau' solves
+ * tau' + c(tau') = tau, where c bounds the rounding error of the floating-point factorisation (Demmel; Higham,
+ * Thm 10.3, with u = 2^-52 and inner products of at most Zdim terms, plus the rounding of the shift and an underflow
+ * term); every operation of c is rounded up.  If every pivot is positive, lambda_max(Z) <= tau' + c(tau') = bound[q]
+ * <= tau[q] is PROVEN for the FP64 Z the library emits (all output formats hold the same bits).  The error of
+ * assembling that Z from gamma is not bounded here -- the reference's eigmax also runs on a floating-point Z.
+ *   tau[q * tau_stride]   0 = one tau for every query; must be finite
+ *   certified[q]          1: lambda_max(Z_q) <= bound[q] <= tau_q;  0: no statement (a result, not an error)
+ *   bound[q]              tau' + c(tau'), written for every query
+ *   fail_index[q]         0-based Z index of the first pivot that was not positive, in elimination order; -1 if none
+ *                         (with nnsdp_cliques it names the clique, hence the layer, where the LMI breaks)
+ *   min_pivot[q]          (may be NULL) the smallest pivot computed: the failing one for an uncertified query
+ * The call runs the emitter: afterwards the ring slots hold factors and are zeroed again by the next pass, as after
+ * nnsdp_batch_ring_reset.  NNSDP_ERR_STATE before nnsdp_batch_prepare; NNSDP_ERR_ARG for packed, dense-Z and
+ * bounds-only batches.  Blocking. */
+int32_t nnsdp_batch_certify(nnsdp_batch* batch, const double* tau, int64_t tau_stride, int32_t* certified,
+                            double* bound, int64_t* fail_index, double* min_pivot);
+/* The elimination plan of nnsdp_batch_certify (host only): 6 int64 per front (= clique, in order) {out_off, n, npriv,
+ * g0, lead, tail}: the block Z[C_k, C_k] at out_off doubles of a query's blocks output, n = |C_k|; local indices
+ * [0, npriv) are eliminated in this front and are the Z indices g0 .. g0 + npriv - 1; the Schur complement of front k-1
+ * replaces local [0, lead) and [n - tail, n) of front k.  NNSDP_ERR_ASSERT if a layout fact the factorisation relies on
+ * does not hold.  fronts_out == NULL queries the count. */
+int32_t nnsdp_certify_plan(int64_t K, const int64_t* xdims, int64_t beta, int64_t max_fronts, int64_t* fronts_out,
+                           int64_t* nfronts);
+
 /* ---- affine-coefficient mode (SURVEY.md 8f-1) ---------------------------------------------
  * Z(gamma) = Z0 + sum_v gamma_v Z_v for ONE query, restricted to the upper triangle of the clique
  * cover, as COO triplets -- the data from which `@constraint(model, Z .== Zksum)`

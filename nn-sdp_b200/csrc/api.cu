@@ -8,6 +8,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <cmath>
 #include <condition_variable>
 #include <deque>
 #include <functional>
@@ -233,6 +234,8 @@ struct nnsdp_batch {
   std::vector<int64_t> bulk_entries;     // K: output entries of those strips
   int64_t pass_entries = 0;              // entries every query of a pass stores (strips, windows, edges, band)
   std::vector<BulkItem> sel;             // the (slot, block) pairs of the current pass
+  std::vector<CholFront> chol;           // elimination plan of nnsdp_batch_certify (built on first use)
+  DevBuf d_chol;
   nnsdp_sizes sz{};
   PlanHost plan;
   DevBuf d_tiles, d_strips, d_bulk, d_mats, d_panel, d_goff, d_ldG;
@@ -298,7 +301,7 @@ struct nnsdp_batch {
     spans.clear();
   }
   std::vector<DevBuf*> all_bufs() {
-    return {&d_bands, &d_tmaps, &d_tmap_ok, &d_tiles, &d_strips, &d_bulk, &d_mats, &d_panel, &d_goff, &d_ldG, &x1min, &x1max, &ymin, &ymax, &smin, &smax,
+    return {&d_bands, &d_tmaps, &d_tmap_ok, &d_tiles, &d_strips, &d_bulk, &d_mats, &d_panel, &d_goff, &d_ldG, &d_chol, &x1min, &x1max, &ymin, &ymax, &smin, &smax,
             &gin, &gbnd, &gsec, &outS, &outvec, &outinvP, &gout, &xmin, &xmax, &acxmin, &acxmax,
             &smin_c, &smax_c, &d11, &Md, &T0, &Bt, &u, &aff, &part, &act, &cnt, &Z11, &Z1K, &U,
             &gram, &ringbuf, &flags, &cr_rowsA, &cr_rowsB, &cr_bias, &cr_prel, &cr_preu, &cr_du, &cr_bu, &cr_dl};
@@ -377,7 +380,7 @@ int32_t check_flags(nnsdp_batch* b, const char* where) {
 extern "C" {
 
 const char* nnsdp_last_error(void) { return g_err.c_str(); }
-int32_t nnsdp_version(void) { return 101; }
+int32_t nnsdp_version(void) { return 102; }
 
 int32_t nnsdp_device_count(int32_t* count) {
   NN_CHECK(count != nullptr, NNSDP_ERR_ARG, "count is NULL");
@@ -2401,6 +2404,149 @@ extern "C" int32_t nnsdp_batch_lambda_max_ex(nnsdp_batch* b, int32_t max_iters, 
 extern "C" int32_t nnsdp_batch_lambda_max(nnsdp_batch* b, int32_t max_iters, double tol, double* lam_max,
                                           int32_t* iters_out) {
   return nnsdp_batch_lambda_max_ex(b, max_iters, tol, lam_max, iters_out, nullptr, nullptr);
+}
+
+// ---------------------------------------------------------------------------------------------
+// Sound certificate eigmax(Z) <= tau (DESIGN.md section 9): multifrontal Cholesky of tau' I - Z with a margin for its
+// rounding error.  Every host operation of the margin is rounded up (nextafter after round-to-nearest).
+// ---------------------------------------------------------------------------------------------
+namespace {
+
+double up(double x) { return std::nextafter(x, INFINITY); }
+double dn(double x) { return std::nextafter(x, -INFINITY); }
+
+// c(tau') for a Z with Zdim rows whose diagonal has computed sum trZ, sum of magnitudes sabs, largest magnitude mabs
+double certify_margin(double tp, int64_t Zdim, double trZ, double sabs, double mabs) {
+  const double u = 0x1p-52, eta = 0x1p-1074, n = (double)Zdim;
+  const double nu = up((n + 1) * u);
+  const double gam = up(nu / dn(1.0 - nu));
+  const double coef = up(up(gam / dn(1.0 - gam)) + u);
+  // tr(fl(tau' I - Z)) <= tau' Zdim - trZ + 2 (Zdim + 2) u (|tau'| Zdim + sabs): the shift and the device sum rounded
+  const double err = up(up(2.0 * (n + 2) * u) * up(up(fabs(tp) * n) + sabs));
+  const double tr = std::max(0.0, up(up(up(tp * n) - trZ) + err));
+  // underflow: every operation of an entry may add eta; at most Zdim + 2 of them, amplified by a pivot <= 2 + max diag
+  const double uf = up(up(2.0 * n * (n + 2)) * up(up(2.0 + up(fabs(tp) + mabs)) * 2.0) * eta);
+  return up(up(coef * tr) + uf);
+}
+
+// the largest tau' (found by a short descent) whose certified bound tau' + c(tau') rounds up to at most tau
+double certify_shift(double tau, int64_t Zdim, double trZ, double sabs, double mabs, double* bound) {
+  double tp = tau;
+  for (int it = 0; it < 200; ++it) {
+    const double bnd = up(tp + certify_margin(tp, Zdim, trZ, sabs, mabs));
+    if (bnd <= tau) {
+      *bound = bnd;
+      return tp;
+    }
+    tp = dn(tp - std::max(bnd - tau, fabs(tp) * 0x1p-50));
+  }
+  *bound = INFINITY;  // not reached for finite inputs
+  return -INFINITY;
+}
+
+}  // namespace
+
+extern "C" int32_t nnsdp_certify_plan(int64_t K, const int64_t* xdims, int64_t beta, int64_t max_fronts,
+                                      int64_t* fronts_out, int64_t* nfronts) {
+  NN_CHECK(nfronts != nullptr, NNSDP_ERR_ARG, "NULL argument");
+  Shape sh;
+  NN_TRY(shape_from_xdims(K, xdims, &sh));
+  nnsdp_sizes sz;
+  NN_TRY(fill_sizes(sh, beta, &sz));
+  std::vector<CliqueRanges> mats;
+  NN_TRY(format_mats(sh, beta, NNSDP_FORMAT_BLOCKS, &mats));
+  std::vector<CholFront> fr;
+  NN_TRY(build_chol_plan(sh, mats, &fr));
+  *nfronts = (int64_t)fr.size();
+  if (!fronts_out) return NNSDP_OK;
+  NN_CHECK(max_fronts >= (int64_t)fr.size(), NNSDP_ERR_ARG, "max_fronts = %lld < %lld fronts", (long long)max_fronts,
+           (long long)fr.size());
+  for (size_t k = 0; k < fr.size(); ++k) {
+    int64_t* o = fronts_out + 6 * k;
+    o[0] = fr[k].out_off;
+    o[1] = fr[k].n;
+    o[2] = fr[k].npriv;
+    o[3] = fr[k].g0;
+    o[4] = fr[k].lead;
+    o[5] = fr[k].tail;
+  }
+  return NNSDP_OK;
+}
+
+extern "C" int32_t nnsdp_batch_certify(nnsdp_batch* b, const double* tau, int64_t tau_stride, int32_t* certified,
+                                       double* bound, int64_t* fail_index, double* min_pivot) {
+  NN_CHECK(b && tau && certified && bound && fail_index, NNSDP_ERR_ARG, "NULL argument");
+  NN_CHECK(b->ring > 0 && !b->dense && !b->packed, NNSDP_ERR_ARG,
+           "nnsdp_batch_certify needs a batch in NNSDP_FORMAT_BLOCKS with ring_queries > 0");
+  NN_CHECK(tau_stride >= 0, NNSDP_ERR_ARG, "tau_stride must be >= 0");
+  NN_CHECK(b->prepared, NNSDP_ERR_STATE, "nnsdp_batch_certify before nnsdp_batch_prepare");
+  for (int64_t q = 0; q < b->Q; ++q)
+    NN_CHECK(std::isfinite(tau[q * tau_stride]), NNSDP_ERR_ARG, "tau of query %lld is not finite", (long long)q);
+  NN_CUDA(cudaSetDevice(b->dev));
+  const Shape& sh = b->net->sh;
+  if (b->chol.empty()) {
+    std::vector<CholFront> fr;
+    NN_TRY(build_chol_plan(sh, b->mats_host, &fr));
+    for (size_t k = 0; k < fr.size(); ++k)
+      NN_CHECK(fr[k].out_off == b->plan.mats[k].out_off, NNSDP_ERR_ASSERT, "certify plan: front %d misplaced", (int)k);
+    NN_TRY(upload(b->d_chol, fr.data(), fr.size() * sizeof(CholFront), b->st));
+    b->chol = fr;
+  }
+  const int nf = (int)b->chol.size();
+  const int64_t R = b->ring, per = b->plan.per_query_doubles;
+  DevBuf dtaup, dstats, dfailed, dfidx, dminp;
+  struct Rel {
+    std::vector<DevBuf*> v;
+    ~Rel() { for (DevBuf* x : v) x->release(); }
+  } rel{{&dtaup, &dstats, &dfailed, &dfidx, &dminp}};
+  NN_TRY(dtaup.ensure((size_t)R * 8));
+  NN_TRY(dstats.ensure((size_t)R * 24));
+  NN_TRY(dfailed.ensure((size_t)R * 4));
+  NN_TRY(dfidx.ensure((size_t)R * 8));
+  NN_TRY(dminp.ensure((size_t)R * 8));
+  std::vector<double> hstats(3 * R), htaup(R), hminp(R);
+  std::vector<int> hfailed(R);
+  std::vector<long long> hfidx(R);
+  double* ring = b->ringbuf.as<double>();
+  for (int64_t q0 = 0; q0 < b->Q; q0 += R) {
+    const int nq = (int)std::min<int64_t>(R, b->Q - q0);
+    NN_TRY(nnsdp_batch_emit(b, q0, nq));
+    b->ring_zeroed = 0;  // the slots will hold factors: the next pass zeroes them again and stores every entry
+    launch_chol_trace(ring, per, b->d_chol.as<CholFront>(), nf, nq, dstats.as<double>(), b->st);
+    NN_CUDA(cudaMemcpyAsync(hstats.data(), dstats.p, (size_t)nq * 24, cudaMemcpyDeviceToHost, b->st));
+    NN_CUDA(cudaStreamSynchronize(b->st));
+    for (int i = 0; i < nq; ++i) {
+      htaup[i] = certify_shift(tau[(q0 + i) * tau_stride], sh.Zdim, hstats[3 * i], hstats[3 * i + 1], hstats[3 * i + 2],
+                               &bound[q0 + i]);
+      hfailed[i] = 0;
+      hfidx[i] = -1;
+      hminp[i] = INFINITY;
+    }
+    NN_CUDA(cudaMemcpyAsync(dtaup.p, htaup.data(), (size_t)nq * 8, cudaMemcpyHostToDevice, b->st));
+    NN_CUDA(cudaMemcpyAsync(dfailed.p, hfailed.data(), (size_t)nq * 4, cudaMemcpyHostToDevice, b->st));
+    NN_CUDA(cudaMemcpyAsync(dfidx.p, hfidx.data(), (size_t)nq * 8, cudaMemcpyHostToDevice, b->st));
+    NN_CUDA(cudaMemcpyAsync(dminp.p, hminp.data(), (size_t)nq * 8, cudaMemcpyHostToDevice, b->st));
+    int launches = 1;
+    for (int k = 0; k < nf; ++k) {
+      const CholFront& f = b->chol[k];
+      launches += launch_chol_front_init(ring, per, f, k > 0 ? &b->chol[k - 1] : nullptr, nq, dtaup.as<double>(),
+                                         dfailed.as<int>(), b->st);
+      for (int j0 = 0; j0 < f.npriv; j0 += CHOL_NB)
+        launches += launch_chol_panel(ring, per, f, j0, std::min(CHOL_NB, f.npriv - j0), nq, dfailed.as<int>(),
+                                      dfidx.as<long long>(), dminp.as<double>(), b->st);
+    }
+    NN_CUDA(cudaGetLastError());
+    NN_CUDA(cudaMemcpyAsync(hfailed.data(), dfailed.p, (size_t)nq * 4, cudaMemcpyDeviceToHost, b->st));
+    NN_CUDA(cudaMemcpyAsync(hfidx.data(), dfidx.p, (size_t)nq * 8, cudaMemcpyDeviceToHost, b->st));
+    NN_CUDA(cudaMemcpyAsync(hminp.data(), dminp.p, (size_t)nq * 8, cudaMemcpyDeviceToHost, b->st));
+    NN_CUDA(cudaStreamSynchronize(b->st));
+    for (int i = 0; i < nq; ++i) {
+      certified[q0 + i] = hfailed[i] ? 0 : 1;
+      fail_index[q0 + i] = hfidx[i];
+      if (min_pivot) min_pivot[q0 + i] = hminp[i];
+    }
+  }
+  return NNSDP_OK;
 }
 
 // -----------------------------------------------------------------------------------------

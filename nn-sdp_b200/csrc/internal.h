@@ -240,6 +240,21 @@ int32_t build_gather_plan(const Shape& sh, int64_t beta, const std::vector<Cliqu
                           const PlanHost& plan, GatherPlan* gp);
 
 // ---------------------------------------------------------------------------------
+// elimination plan of the certificate (nnsdp_batch_certify): multifrontal Cholesky of tau' I - Z along the path of
+// cliques, in the natural order.  Front k is the clique block Z[C_k, C_k] of the NNSDP_FORMAT_BLOCKS output, in place.
+// Its private indices (whose last clique is k) are local [0, npriv) and eliminated there; the Schur complement on the
+// remaining local indices [npriv, n) replaces front k+1's entries on local [0, lead) and [n_{k+1} - tail, n_{k+1}).
+// ---------------------------------------------------------------------------------
+struct CholFront {
+  long long out_off;  // doubles of Z[C_k, C_k] inside one query's output (leading dimension n)
+  long long g0;       // global z index of local index 0 = the first private index; private ones are contiguous
+  int n, npriv;
+  int lead, tail;     // front k > 0: entries taken over from front k-1's Schur complement (0 and 0 for front 0)
+};
+// Builds the plan from the blocks-format clique ranges and checks every layout fact it relies on (NNSDP_ERR_ASSERT).
+int32_t build_chol_plan(const Shape& sh, const std::vector<CliqueRanges>& mats, std::vector<CholFront>* fronts);
+
+// ---------------------------------------------------------------------------------
 // device-side descriptors (passed by value to kernels)
 // ---------------------------------------------------------------------------------
 struct NetDev {
@@ -457,6 +472,19 @@ int launch_crown_concretize(const double* rowsL, const double* rowsU, long long 
                             int nrows, int Rs, int row0, int Qc, int n0, const double* x1min, long long s_min,
                             const double* x1max, long long s_max, int q_first, const double* bias, double* out_lo,
                             double* out_hi, long long out_stride, int postprocess, cudaStream_t st);
+
+// certificate kernels (kernels_chol.cu) on ring slots 0 .. nq-1 (slot stride `per` doubles)
+constexpr int CHOL_NB = 32;  // panel width
+// stats[3 s + {0, 1, 2}] = sum, sum of |.|, max |.| of the diagonal of Z in slot s (every index once)
+int launch_chol_trace(const double* ring, long long per, const CholFront* fronts, int nfronts, int nq, double* stats,
+                      cudaStream_t st);
+// front f := tau' I - Z[C, C] (lower triangle), with the overlap taken from prev's Schur complement (prev == null: none)
+int launch_chol_front_init(double* ring, long long per, const CholFront& f, const CholFront* prev, int nq,
+                           const double* taup, const int* failed, cudaStream_t st);
+// columns [j0, j0 + w) of front f: Cholesky of the diagonal block (pivots checked), TRSM of the rows below, SYRK update
+// of the trailing lower triangle on the FP64 tensor cores.  A query whose pivot is not positive stops there.
+int launch_chol_panel(double* ring, long long per, const CholFront& f, int j0, int w, int nq, int* failed,
+                      long long* fail_index, double* min_pivot, cudaStream_t st);
 
 // band jobs (in-place band of the DIAG ranges, BAND cells of packed records) for queries [q0, q0+nq); after the fill kernel
 int launch_emit_band(const NetDev& net, const BatchDev& b, const GramDev& g, const BandDev* bands, int nbands,

@@ -117,6 +117,72 @@ int32_t fill_sizes(const Shape& sh, int64_t beta, nnsdp_sizes* s) {
   return NNSDP_OK;
 }
 
+// The layout facts are checked, not assumed: every index lies in some clique; the private indices of clique k (whose
+// last clique is k) are a leading, globally contiguous range of its local order; everything else of clique k lies in
+// clique k+1, at local [0, lead) in order and at the tail [n_{k+1} - tail, n_{k+1}); the last clique is all private; and
+// the indices a front does not take over (where its diagonal is shifted) cover 0 .. Zdim-1 exactly once.
+int32_t build_chol_plan(const Shape& sh, const std::vector<CliqueRanges>& mats, std::vector<CholFront>* fronts) {
+  const int p = (int)mats.size();
+  NN_CHECK(p >= 1, NNSDP_ERR_ASSERT, "certify plan: no clique");
+  std::vector<std::vector<int64_t>> idx(p);
+  std::vector<int> owner(sh.Zdim, -1);
+  for (int k = 0; k < p; ++k) {
+    for (int s = 0; s < mats[k].nseg; ++s)
+      for (int64_t g = mats[k].lo[s]; g <= mats[k].hi[s]; ++g) idx[k].push_back(g);
+    for (int64_t g : idx[k]) {
+      NN_CHECK(g >= 0 && g < sh.Zdim, NNSDP_ERR_ASSERT, "certify plan: index %lld outside Z", (long long)g);
+      owner[g] = k;
+    }
+  }
+  for (int64_t g = 0; g < sh.Zdim; ++g)
+    NN_CHECK(owner[g] >= 0, NNSDP_ERR_ASSERT, "certify plan: index %lld lies in no clique", (long long)g);
+  fronts->assign(p, CholFront{});
+  std::vector<uint8_t> shifted(sh.Zdim, 0);
+  long long off = 0;
+  for (int k = 0; k < p; ++k) {
+    CholFront& f = (*fronts)[k];
+    const std::vector<int64_t>& c = idx[k];
+    f.out_off = off;
+    f.n = (int)c.size();
+    off += (long long)f.n * f.n;
+    int np = 0;
+    while (np < f.n && owner[c[np]] == k) ++np;
+    f.npriv = np;
+    f.g0 = c[0];
+    for (int i = 0; i < f.n; ++i) {
+      NN_CHECK((owner[c[i]] == k) == (i < np), NNSDP_ERR_ASSERT,
+               "certify plan: the private indices of clique %d are not a leading range", k + 1);
+      if (i < np)
+        NN_CHECK(c[i] == f.g0 + i, NNSDP_ERR_ASSERT, "certify plan: private indices of clique %d not contiguous", k + 1);
+    }
+    NN_CHECK(np >= 1, NNSDP_ERR_ASSERT, "certify plan: clique %d has no private index", k + 1);
+    NN_CHECK(k + 1 < p || np == f.n, NNSDP_ERR_ASSERT, "certify plan: the last clique is not all private");
+    if (k > 0) {  // map front k-1's Schur complement into this front
+      const CholFront& pf = (*fronts)[k - 1];
+      const std::vector<int64_t>& pc = idx[k - 1];
+      const int ns = pf.n - pf.npriv;
+      const int seg1 = (int)(mats[k - 1].hi[0] - mats[k - 1].lo[0] + 1);
+      f.lead = seg1 - pf.npriv;
+      f.tail = ns - f.lead;
+      NN_CHECK(f.lead >= 0 && f.tail >= 0 && f.lead + f.tail <= f.n, NNSDP_ERR_ASSERT,
+               "certify plan: separator of cliques %d, %d does not fit", k, k + 1);
+      for (int s = 0; s < ns; ++s) {
+        const int li = s < f.lead ? s : f.n - (ns - s);
+        NN_CHECK(c[li] == pc[pf.npriv + s], NNSDP_ERR_ASSERT,
+                 "certify plan: index %lld of clique %d is not at its place in clique %d", (long long)pc[pf.npriv + s], k,
+                 k + 1);
+      }
+    }
+    for (int i = f.lead; i < f.n - f.tail; ++i) {
+      NN_CHECK(!shifted[c[i]], NNSDP_ERR_ASSERT, "certify plan: diagonal entry %lld shifted twice", (long long)c[i]);
+      shifted[c[i]] = 1;
+    }
+  }
+  for (int64_t g = 0; g < sh.Zdim; ++g)
+    NN_CHECK(shifted[g], NNSDP_ERR_ASSERT, "certify plan: diagonal entry %lld never shifted", (long long)g);
+  return NNSDP_OK;
+}
+
 namespace {
 
 struct Piece {

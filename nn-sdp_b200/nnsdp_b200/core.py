@@ -176,6 +176,21 @@ def plan_panel(xdims: Sequence[int], beta: int, dense: int = 0) -> np.ndarray:
     return out
 
 
+CERTIFY_PLAN_FIELDS = ("out_off", "n", "npriv", "g0", "lead", "tail")
+
+
+def certify_plan(xdims: Sequence[int], beta: int) -> np.ndarray:
+    """The elimination plan of Batch.certify as an (nfronts, 6) int64 array (columns: CERTIFY_PLAN_FIELDS).  Raises
+    NnsdpError(ERR_ASSERT) if a layout fact of the multifrontal factorisation does not hold.  Host only."""
+    K = len(xdims) - 1
+    xd = (L.c_i64 * (K + 1))(*[int(x) for x in xdims])
+    n = L.c_i64(0)
+    L.check(L.lib.nnsdp_certify_plan(K, xd, beta, 0, None, C.byref(n)))
+    out = np.zeros((int(n.value), 6), dtype=np.int64)
+    L.check(L.lib.nnsdp_certify_plan(K, xd, beta, int(n.value), out.ctypes.data_as(L.c_i64p), C.byref(n)))
+    return out
+
+
 def plan_tiles(xdims: Sequence[int], beta: int, dense: bool = False) -> np.ndarray:
     """The emission plan's tile list as an (ntiles, 11) int32 array (columns: TILE_FIELDS); host only."""
     K = len(xdims) - 1
@@ -565,6 +580,43 @@ class Batch:
             return lam, its, resid, conv
         L.check(st)
         return lam, its
+
+    def certify(self, tau):
+        """Sound certificate lambda_max(Z_q) <= tau_q (nnsdp_batch_certify); needs bounds + prepare.  tau: a scalar or
+        one value per query.  Returns (certified, bound, fail_index, min_pivot): certified[q] = 1 proves
+        lambda_max(Z_q) <= bound[q] <= tau_q; fail_index[q] is the 0-based Z index of the first non-positive pivot or -1."""
+        t = np.ascontiguousarray(np.atleast_1d(np.asarray(tau, dtype=np.float64)))
+        if t.size not in (1, self.Q):
+            raise ValueError(f"tau has {t.size} values for {self.Q} queries")
+        cert = np.zeros(self.Q, dtype=np.int32)
+        bound = np.zeros(self.Q)
+        fidx = np.zeros(self.Q, dtype=np.int64)
+        minp = np.zeros(self.Q)
+        L.check(L.lib.nnsdp_batch_certify(self._h, _dp(t), 0 if t.size == 1 else 1, cert.ctypes.data_as(C.POINTER(L.c_i32)),
+                                          _dp(bound), fidx.ctypes.data_as(L.c_i64p), _dp(minp)))
+        return cert, bound, fidx, minp
+
+    def lambda_max_bracket(self, max_iters: int = 300, tol: float = 1e-10, rel: float = 1e-9, growth: float = 10.0,
+                           max_tries: int = 12, scale=None):
+        """A sound interval lo <= lambda_max(Z_q) <= hi for every query: lo is the Lanczos Ritz value (always a lower
+        bound, converged or not), hi the bound of certify at tau = lo + rel * scale * growth^t for t = 0, 1, ... until the
+        query certifies (hi = inf if it never does within max_tries).  scale (per query or scalar) defaults to
+        max(|lo|, resid).  Returns (lo, hi, certified)."""
+        lo, _, resid, _ = self.lambda_max(max_iters=max_iters, tol=tol, full=True)
+        s = np.maximum(np.abs(lo), resid) if scale is None else np.broadcast_to(np.asarray(scale, dtype=float), lo.shape)
+        s = np.maximum(s, np.finfo(float).tiny)
+        hi = np.full(self.Q, np.inf)
+        done = np.zeros(self.Q, dtype=bool)
+        step = rel * s
+        for _ in range(max_tries):
+            cert, bound, _, _ = self.certify(lo + step)
+            new = (cert == 1) & ~done
+            hi[new] = bound[new]
+            done |= new
+            if done.all():
+                break
+            step = step * growth
+        return lo, hi, done.astype(np.int32)
 
     def gather_stats(self) -> dict:
         a, t, z, u = L.c_i64(0), L.c_i64(0), L.c_i64(0), L.c_i32(0)
