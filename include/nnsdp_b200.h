@@ -400,6 +400,13 @@ int32_t nnsdp_batch_lambda_max(nnsdp_batch* batch, int32_t max_iters, double tol
  * bounds-only batches.  Blocking. */
 int32_t nnsdp_batch_certify(nnsdp_batch* batch, const double* tau, int64_t tau_stride, int32_t* certified,
                             double* bound, int64_t* fail_index, double* min_pivot);
+/* nnsdp_batch_certify with the other side: lower[q] (may be NULL) is a PROVEN lower bound of lambda_max(Z_q) for a
+ * query that was not certified, from the failed factorisation of fl(tau' I - Z) (Demmel's success condition; Higham,
+ * Thm 10.7, with the same u and n as the margin): lambda_max(Z_q) >= tau' - n g/(1 - n g) max|a_ii| - u max|a_ii| -
+ * underflow, g = gamma_{n+1}.  -inf for a certified query, and when the factorisation may have overflowed (a large
+ * diagonal, or a failing pivot that is not finite). */
+int32_t nnsdp_batch_certify_ex(nnsdp_batch* batch, const double* tau, int64_t tau_stride, int32_t* certified,
+                               double* bound, int64_t* fail_index, double* min_pivot, double* lower);
 /* The elimination plan of nnsdp_batch_certify (host only): 6 int64 per front (= clique, in order) {out_off, n, npriv,
  * g0, lead, tail}: the block Z[C_k, C_k] at out_off doubles of a query's blocks output, n = |C_k|; local indices
  * [0, npriv) are eliminated in this front and are the Z indices g0 .. g0 + npriv - 1; the Schur complement of front k-1

@@ -380,7 +380,7 @@ int32_t check_flags(nnsdp_batch* b, const char* where) {
 extern "C" {
 
 const char* nnsdp_last_error(void) { return g_err.c_str(); }
-int32_t nnsdp_version(void) { return 102; }
+int32_t nnsdp_version(void) { return 103; }
 
 int32_t nnsdp_device_count(int32_t* count) {
   NN_CHECK(count != nullptr, NNSDP_ERR_ARG, "count is NULL");
@@ -2444,6 +2444,26 @@ double certify_shift(double tau, int64_t Zdim, double trZ, double sabs, double m
   return -INFINITY;
 }
 
+// A proven lower bound of lambda_max(Z) after the factorisation of fl(tau' I - Z) failed.  Demmel's success condition
+// (Higham, Thm 10.7): the Cholesky of A = fl(tau' I - Z) runs to completion when lambda_min(D^-1 A D^-1) > n g / (1 - n g)
+// with D = diag(a_ii)^(1/2), g = gamma_{n+1} (u = 2^-52, as in the margin).  A failure therefore gives
+// lambda_min(A) <= n g / (1 - n g) max a_ii (or <= 0 if a diagonal entry is not positive), and A differs from
+// tau' I - Z by the shift's rounding, at most u max|a_ii|.  So lambda_max(Z) >= tau' - rho amax - u amax - underflow.
+// -inf when the factorisation may have overflowed (then a failure proves nothing).
+double certify_lower(double tp, int64_t Zdim, double mabs) {
+  const double u = 0x1p-52, eta = 0x1p-1074, n = (double)Zdim;
+  const double nu = up((n + 1) * u);
+  const double gam = up(nu / dn(1.0 - nu));
+  const double ng = up(n * gam);
+  if (!(ng < 0.5)) return -INFINITY;
+  const double rho = up(ng / dn(1.0 - ng));
+  const double amax = up(up(fabs(tp) + mabs) * up(1.0 + 2.0 * u));   // >= max |fl(tau' - z_ii)|
+  if (!std::isfinite(amax) || !std::isfinite(up(up(4.0 * n) * amax)) || !std::isfinite(tp)) return -INFINITY;
+  const double uf = up(up(2.0 * n * (n + 2)) * up(up(2.0 + amax) * 2.0) * eta);
+  const double m = up(up(up(rho * amax) + up(u * amax)) + uf);
+  return dn(tp - m);
+}
+
 }  // namespace
 
 extern "C" int32_t nnsdp_certify_plan(int64_t K, const int64_t* xdims, int64_t beta, int64_t max_fronts,
@@ -2475,6 +2495,11 @@ extern "C" int32_t nnsdp_certify_plan(int64_t K, const int64_t* xdims, int64_t b
 
 extern "C" int32_t nnsdp_batch_certify(nnsdp_batch* b, const double* tau, int64_t tau_stride, int32_t* certified,
                                        double* bound, int64_t* fail_index, double* min_pivot) {
+  return nnsdp_batch_certify_ex(b, tau, tau_stride, certified, bound, fail_index, min_pivot, nullptr);
+}
+
+extern "C" int32_t nnsdp_batch_certify_ex(nnsdp_batch* b, const double* tau, int64_t tau_stride, int32_t* certified,
+                                          double* bound, int64_t* fail_index, double* min_pivot, double* lower) {
   NN_CHECK(b && tau && certified && bound && fail_index, NNSDP_ERR_ARG, "NULL argument");
   NN_CHECK(b->ring > 0 && !b->dense && !b->packed, NNSDP_ERR_ARG,
            "nnsdp_batch_certify needs a batch in NNSDP_FORMAT_BLOCKS with ring_queries > 0");
@@ -2504,7 +2529,7 @@ extern "C" int32_t nnsdp_batch_certify(nnsdp_batch* b, const double* tau, int64_
   NN_TRY(dfailed.ensure((size_t)R * 4));
   NN_TRY(dfidx.ensure((size_t)R * 8));
   NN_TRY(dminp.ensure((size_t)R * 8));
-  std::vector<double> hstats(3 * R), htaup(R), hminp(R);
+  std::vector<double> hstats(3 * R), htaup(R), hminp(R), hlower(R);
   std::vector<int> hfailed(R);
   std::vector<long long> hfidx(R);
   double* ring = b->ringbuf.as<double>();
@@ -2518,6 +2543,7 @@ extern "C" int32_t nnsdp_batch_certify(nnsdp_batch* b, const double* tau, int64_
     for (int i = 0; i < nq; ++i) {
       htaup[i] = certify_shift(tau[(q0 + i) * tau_stride], sh.Zdim, hstats[3 * i], hstats[3 * i + 1], hstats[3 * i + 2],
                                &bound[q0 + i]);
+      hlower[i] = certify_lower(htaup[i], sh.Zdim, hstats[3 * i + 2]);
       hfailed[i] = 0;
       hfidx[i] = -1;
       hminp[i] = INFINITY;
@@ -2544,6 +2570,8 @@ extern "C" int32_t nnsdp_batch_certify(nnsdp_batch* b, const double* tau, int64_
       certified[q0 + i] = hfailed[i] ? 0 : 1;
       fail_index[q0 + i] = hfidx[i];
       if (min_pivot) min_pivot[q0 + i] = hminp[i];
+      // an infinite or NaN failing pivot means an overflow or a non-finite Z: the failure then proves nothing
+      if (lower) lower[q0 + i] = hfailed[i] && std::isfinite(hminp[i]) ? hlower[i] : -INFINITY;
     }
   }
   return NNSDP_OK;

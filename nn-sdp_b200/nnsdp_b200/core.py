@@ -581,10 +581,12 @@ class Batch:
         L.check(st)
         return lam, its
 
-    def certify(self, tau):
+    def certify(self, tau, lower: bool = False):
         """Sound certificate lambda_max(Z_q) <= tau_q (nnsdp_batch_certify); needs bounds + prepare.  tau: a scalar or
         one value per query.  Returns (certified, bound, fail_index, min_pivot): certified[q] = 1 proves
-        lambda_max(Z_q) <= bound[q] <= tau_q; fail_index[q] is the 0-based Z index of the first non-positive pivot or -1."""
+        lambda_max(Z_q) <= bound[q] <= tau_q; fail_index[q] is the 0-based Z index of the first non-positive pivot or -1.
+        lower=True appends lower (nnsdp_batch_certify_ex): for a query that was not certified, a proven lower bound of
+        lambda_max(Z_q) from the failed factorisation; -inf for a certified one."""
         t = np.ascontiguousarray(np.atleast_1d(np.asarray(tau, dtype=np.float64)))
         if t.size not in (1, self.Q):
             raise ValueError(f"tau has {t.size} values for {self.Q} queries")
@@ -592,31 +594,39 @@ class Batch:
         bound = np.zeros(self.Q)
         fidx = np.zeros(self.Q, dtype=np.int64)
         minp = np.zeros(self.Q)
-        L.check(L.lib.nnsdp_batch_certify(self._h, _dp(t), 0 if t.size == 1 else 1, cert.ctypes.data_as(C.POINTER(L.c_i32)),
-                                          _dp(bound), fidx.ctypes.data_as(L.c_i64p), _dp(minp)))
-        return cert, bound, fidx, minp
+        lo = np.zeros(self.Q)
+        L.check(L.lib.nnsdp_batch_certify_ex(self._h, _dp(t), 0 if t.size == 1 else 1,
+                                             cert.ctypes.data_as(C.POINTER(L.c_i32)), _dp(bound),
+                                             fidx.ctypes.data_as(L.c_i64p), _dp(minp), _dp(lo) if lower else None))
+        return (cert, bound, fidx, minp, lo) if lower else (cert, bound, fidx, minp)
 
     def lambda_max_bracket(self, max_iters: int = 300, tol: float = 1e-10, rel: float = 1e-9, growth: float = 10.0,
                            max_tries: int = 12, scale=None):
-        """A sound interval lo <= lambda_max(Z_q) <= hi for every query: lo is the Lanczos Ritz value (always a lower
-        bound, converged or not), hi the bound of certify at tau = lo + rel * scale * growth^t for t = 0, 1, ... until the
-        query certifies (hi = inf if it never does within max_tries).  scale (per query or scalar) defaults to
-        max(|lo|, resid).  Returns (lo, hi, certified)."""
-        lo, _, resid, _ = self.lambda_max(max_iters=max_iters, tol=tol, full=True)
-        s = np.maximum(np.abs(lo), resid) if scale is None else np.broadcast_to(np.asarray(scale, dtype=float), lo.shape)
+        """A sound interval lo <= lambda_max(Z_q) <= hi for every query, both ends proven by a factorisation of
+        fl(tau' I - Z): hi is the bound of a certified call, lo the lower bound of a failed one (certify(lower=True)).
+        The Lanczos Ritz value r only places the tries: it is not a bound (its rounding error may put it above
+        lambda_max).  The first try is tau = r; then a query still without hi tries r + rel * scale * growth^t, one
+        still without lo tries r - rel * scale * growth^t, t = 0, 1, ..., at most max_tries calls in all.  An end no try
+        proves stays -inf / inf.  scale (per query or scalar) defaults to max(|r|, resid).  Returns (lo, hi, certified),
+        certified = 1 where hi is finite."""
+        r, _, resid, _ = self.lambda_max(max_iters=max_iters, tol=tol, full=True)
+        s = np.maximum(np.abs(r), resid) if scale is None else np.broadcast_to(np.asarray(scale, dtype=float), r.shape)
         s = np.maximum(s, np.finfo(float).tiny)
+        lo = np.full(self.Q, -np.inf)
         hi = np.full(self.Q, np.inf)
-        done = np.zeros(self.Q, dtype=bool)
+        tau = r.copy()
         step = rel * s
         for _ in range(max_tries):
-            cert, bound, _, _ = self.certify(lo + step)
-            new = (cert == 1) & ~done
-            hi[new] = bound[new]
-            done |= new
-            if done.all():
+            cert, bound, _, _, low = self.certify(tau, lower=True)
+            ok = cert == 1
+            hi[ok] = np.minimum(hi[ok], bound[ok])
+            lo[~ok] = np.maximum(lo[~ok], low[~ok])
+            need_hi, need_lo = ~np.isfinite(hi), ~np.isfinite(lo)
+            if not (need_hi | need_lo).any():
                 break
+            tau = np.where(need_hi, r + step, np.where(need_lo, r - step, r))
             step = step * growth
-        return lo, hi, done.astype(np.int32)
+        return lo, hi, np.isfinite(hi).astype(np.int32)
 
     def gather_stats(self) -> dict:
         a, t, z, u = L.c_i64(0), L.c_i64(0), L.c_i64(0), L.c_i32(0)

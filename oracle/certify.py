@@ -47,6 +47,23 @@ def certify_shift(tau, zdim, trz, sabs, mabs):
     return -math.inf, math.inf
 
 
+def certify_lower(tp, zdim, mabs):
+    """Proven lower bound of lambda_max(Z) after the factorisation of fl(tau' I - Z) failed (Demmel's success condition,
+    Higham Thm 10.7; nnsdp_batch_certify_ex).  -inf where the factorisation may have overflowed."""
+    n = float(zdim)
+    nu = _up((n + 1) * U)
+    gam = _up(nu / _dn(1.0 - nu))
+    ng = _up(n * gam)
+    if not ng < 0.5:
+        return -math.inf
+    rho = _up(ng / _dn(1.0 - ng))
+    amax = _up(_up(abs(tp) + mabs) * _up(1.0 + 2.0 * U))
+    if not (math.isfinite(amax) and math.isfinite(_up(_up(4.0 * n) * amax)) and math.isfinite(tp)):
+        return -math.inf
+    uf = _up(_up(2.0 * n * (n + 2)) * _up(_up(2.0 + amax) * 2.0) * ETA)
+    return _dn(tp - _up(_up(_up(rho * amax) + _up(U * amax)) + uf))
+
+
 def front_plan(cliques, zdim):
     """Per front: (npriv, lead, tail) with the layout checks of the device plan."""
     p = len(cliques)
