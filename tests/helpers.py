@@ -68,3 +68,76 @@ def relerr(a, b):
     b = np.asarray(b)
     scale = max(np.abs(b).max(), 1e-300)
     return np.abs(a - b).max() / scale
+
+
+# ---- queries for the entrywise checks (oracle/exact_z.py) ---------------------------------------------------------
+
+def wide_range_net(xdims, seed):
+    """A net whose Gram blocks mix huge and tiny entries: the weight rows of layer k scaled by 2^U{-k_max..k_max}
+    (k_max grows with the layer); the first layer keeps |w|, |b| ≤ 1 (the layer of the subnormal λ of
+    wide_range_query, see the underflow term of exact_z).  Rows 0 and 1 of the last hidden layer are equal up to the
+    sign of the second half of their inputs (the exact cancellation of wide_range_query)."""
+    rng = np.random.default_rng(seed)
+    Ms = []
+    for k, M in enumerate(rand_net(xdims, seed=seed).Ms):
+        M = M.copy()
+        if k == 0:
+            M /= max(1.0, np.abs(M).max())
+            M[:, :-1] *= 2.0 ** -rng.integers(0, 6, M.shape[0])[:, None]
+        else:
+            km = min(4 + 4 * k, 24)
+            M *= 2.0 ** rng.integers(-km, km + 1, M.shape[0])[:, None]
+        Ms.append(M)
+    K = len(xdims) - 1
+    if K >= 3 and xdims[K - 1] >= 2:
+        M, n_in = Ms[K - 2], xdims[K - 2]
+        M[1, :-1] = M[0, :-1] * np.where(np.arange(n_in) < (n_in + 1) // 2, 1.0, -1.0)
+    return o.FeedFwdNet(xdims=list(xdims), Ms=Ms)
+
+
+def wide_range_query(net, beta, kind, rng):
+    """A query (and its QC bounds) whose entries span many binades:
+    - every γ component 2^U(-40, 40); fractional slopes 0 < smin ≤ smax < 1, some neurons stably active (1, 1) with
+      λ = 0 on some of them, some with smin = 0 (d11 = 0: not Gram-active);
+    - on layer 1 a λ = 2⁻¹⁰⁷⁰ (d11 subnormal, Gram-active) and a λ = 2⁻¹⁰⁷⁴ with smin·smax < 1/2 (d11 rounds to 0);
+    - neurons 0 and 1 of the last hidden layer (rows equal up to sign, wide_range_net) with the same d11 are the only
+      Gram-active neurons of their layer: their Gram terms cancel exactly on the mixed entries."""
+    xdims, K = net.xdims, net.K
+    ac, n1 = net.acdim, xdims[0]
+    p2 = lambda n: 2.0 ** rng.uniform(-40, 40, n)
+    ymin = -(2.0 ** rng.uniform(-6, 6, ac))
+    ymax = ymin + 2.0 ** rng.uniform(-6, 6, ac)
+    smin = rng.uniform(0.05, 0.95, ac)
+    smax = np.minimum(smin + rng.uniform(0.0, 0.5, ac), 0.97)
+    state = rng.random(ac)
+    smin[state < 0.15], smax[state < 0.15] = 1.0, 1.0            # stably active
+    smin[state > 0.85] = 0.0                                      # d11 = 0
+    gsec = p2(o.sector_lambda_dim(ac, beta) + 2 * ac)
+    lam = gsec[:ac]
+    lam[(state < 0.15) & (rng.random(ac) < 0.5)] = 0.0           # λ = 0 on stably active neurons
+    if xdims[1] >= 2:
+        smin[0], smax[0], lam[0] = 0.5, 0.5, 2.0 ** -1070         # d11 = -2^-1071
+        smin[1], smax[1], lam[1] = 0.5, 0.75, 2.0 ** -1074        # p λ = 0.375 · 2^-1074 rounds to 0
+    if K >= 3 and xdims[K - 1] >= 2:
+        j1 = ac - xdims[K - 1]
+        smin[j1:] = 0.0
+        smin[j1:j1 + 2], smax[j1:j1 + 2], lam[j1:j1 + 2] = 0.25, 0.5, p2(1)[0]
+    q = rand_query(net, beta, rng, kind=kind, centre=rng.uniform(-1, 1, n1), radius=0.5)
+    q.gin, q.gbnd, q.gsec = p2(n1), p2(ac), gsec
+    if q.gout is not None:
+        q.gout = p2(1)
+    return q, (ymin, ymax, smin, smax)
+
+
+def wide_range_case(xdims, beta, kind, seed):
+    net = wide_range_net(xdims, seed)
+    q, bounds = wide_range_query(net, beta, kind, np.random.default_rng(seed + 1000))
+    return net, q, bounds
+
+
+def assert_meets(R, Z, what=""):
+    ok, ratio = R.check(Z)
+    if not ok.all():
+        i, c = np.unravel_index(np.argmax(np.where(ok, 0, ratio)), ok.shape)
+        raise AssertionError(f"{what}: {int((~ok).sum())} entries break the bound; worst Z[{R.rows[i]},{c}] = "
+                             f"{Z[i, c]!r}, |err| / bound = {ratio[i, c]:.3g}, abs = {R.abs[i, c]:.3g}, N = {R.N[i, c]}")
