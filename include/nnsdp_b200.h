@@ -415,6 +415,33 @@ int32_t nnsdp_batch_certify_ex(nnsdp_batch* batch, const double* tau, int64_t ta
 int32_t nnsdp_certify_plan(int64_t K, const int64_t* xdims, int64_t beta, int64_t max_fronts, int64_t* fronts_out,
                            int64_t* nfronts);
 
+/* ---- the certificate for the exact Z(gamma) (DESIGN.md section 9) ---------------------------------------------
+ * Z(gamma) is the matrix of exact arithmetic built from the same FP64 data as the emitted Z_dev: weights, biases, the
+ * box, gamma, the output QC and the QC bounds ymin / ymax / smin / smax AS THE BATCH HOLDS THEM (given, or computed by
+ * nnsdp_batch_bounds; nnsdp_batch_get_bounds returns them).  Whether those bounds are themselves sound is not
+ * addressed here.  Entrywise |Z_dev[r,c] - Z(gamma)[r,c]| <= gamma_N abs[r,c] + N 2^-1074 (DESIGN.md section 2), abs
+ * being the sum of the absolute values of the entry's monomials and N <= Nmax; hence, E being symmetric,
+ * ||Z_dev - Z(gamma)||_2 <= ||.||_inf <= e_q = up(gamma_Nmax max_r s_q[r]) + up(Zdim Nmax 2^-1074 F_q), with
+ * s_q[r] >= sum_c abs[r,c] computed on the device with every operation rounded up, and F_q the underflow factor of
+ * DESIGN.md section 9.  So lambda_max(Z_dev) - e_q <= lambda_max(Z(gamma)) <= lambda_max(Z_dev) + e_q.
+ *
+ * nnsdp_batch_assembly_error: err[q] = e_q (+inf when an input or an intermediate is not finite); abs_rowsum (may be
+ * NULL) receives s_q, Zdim doubles per query (query q at q * Zdim).  Any output format; emits nothing.
+ * NNSDP_ERR_ARG for bounds-only batches, NNSDP_ERR_STATE before nnsdp_batch_prepare.  Blocking. */
+int32_t nnsdp_batch_assembly_error(nnsdp_batch* batch, double* err, double* abs_rowsum);
+/* Nmax of e_q for a net of these layer widths, beta and output kind (host only): an upper bound of the monomial count
+ * of every entry of Z plus 6 (oracle/exact_z.py's N). */
+int32_t nnsdp_assembly_error_nmax(int64_t K, const int64_t* xdims, int64_t beta, int32_t out_kind, int64_t* nmax);
+/* nnsdp_batch_certify_ex for Z(gamma): e_q first, then the factorisation at tau_dev = the largest double <= tau - e_q.
+ * bound[q] = the smallest double >= bound_dev + e_q, lower[q] = the largest double <= lower_dev - e_q (-inf wherever
+ * lower_dev is).  certified[q] = 1 PROVES lambda_max(Z(gamma)) <= bound[q] <= tau_q; 0 with a finite lower proves
+ * lambda_max(Z(gamma)) >= lower[q].  Where e_q = +inf no factorisation runs: certified = 0, bound = +inf, lower = -inf,
+ * fail_index = -1, min_pivot = +inf.  assembly_err (may be NULL) receives e_q; lower and min_pivot may be NULL.
+ * Same arguments, checks and side effects on the ring as nnsdp_batch_certify_ex, whose results it does not change. */
+int32_t nnsdp_batch_certify_gamma(nnsdp_batch* batch, const double* tau, int64_t tau_stride, int32_t* certified,
+                                  double* bound, int64_t* fail_index, double* min_pivot, double* lower,
+                                  double* assembly_err);
+
 /* ---- affine-coefficient mode (SURVEY.md 8f-1) ---------------------------------------------
  * Z(gamma) = Z0 + sum_v gamma_v Z_v for ONE query, restricted to the upper triangle of the clique
  * cover, as COO triplets -- the data from which `@constraint(model, Z .== Zksum)`

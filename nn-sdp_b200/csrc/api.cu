@@ -236,6 +236,7 @@ struct nnsdp_batch {
   std::vector<BulkItem> sel;             // the (slot, block) pairs of the current pass
   std::vector<CholFront> chol;           // elimination plan of nnsdp_batch_certify (built on first use)
   DevBuf d_chol;
+  DevBuf ze_netv, ze_g, ze_rows, ze_part, ze_io, ze_err;  // nnsdp_batch_assembly_error (allocated on first use)
   nnsdp_sizes sz{};
   PlanHost plan;
   DevBuf d_tiles, d_strips, d_bulk, d_mats, d_panel, d_goff, d_ldG;
@@ -301,7 +302,7 @@ struct nnsdp_batch {
     spans.clear();
   }
   std::vector<DevBuf*> all_bufs() {
-    return {&d_bands, &d_tmaps, &d_tmap_ok, &d_tiles, &d_strips, &d_bulk, &d_mats, &d_panel, &d_goff, &d_ldG, &d_chol, &x1min, &x1max, &ymin, &ymax, &smin, &smax,
+    return {&d_bands, &d_tmaps, &d_tmap_ok, &d_tiles, &d_strips, &d_bulk, &d_mats, &d_panel, &d_goff, &d_ldG, &d_chol, &ze_netv, &ze_g, &ze_rows, &ze_part, &ze_io, &ze_err, &x1min, &x1max, &ymin, &ymax, &smin, &smax,
             &gin, &gbnd, &gsec, &outS, &outvec, &outinvP, &gout, &xmin, &xmax, &acxmin, &acxmax,
             &smin_c, &smax_c, &d11, &Md, &T0, &Bt, &u, &aff, &part, &act, &cnt, &Z11, &Z1K, &U,
             &gram, &ringbuf, &flags, &cr_rowsA, &cr_rowsB, &cr_bias, &cr_prel, &cr_preu, &cr_du, &cr_bu, &cr_dl};
@@ -2493,13 +2494,9 @@ extern "C" int32_t nnsdp_certify_plan(int64_t K, const int64_t* xdims, int64_t b
   return NNSDP_OK;
 }
 
-extern "C" int32_t nnsdp_batch_certify(nnsdp_batch* b, const double* tau, int64_t tau_stride, int32_t* certified,
-                                       double* bound, int64_t* fail_index, double* min_pivot) {
-  return nnsdp_batch_certify_ex(b, tau, tau_stride, certified, bound, fail_index, min_pivot, nullptr);
-}
-
-extern "C" int32_t nnsdp_batch_certify_ex(nnsdp_batch* b, const double* tau, int64_t tau_stride, int32_t* certified,
-                                          double* bound, int64_t* fail_index, double* min_pivot, double* lower) {
+// The arguments of nnsdp_batch_certify_ex and nnsdp_batch_certify_gamma (the same checks for both).
+static int32_t certify_check(nnsdp_batch* b, const double* tau, int64_t tau_stride, const int32_t* certified,
+                             const double* bound, const int64_t* fail_index) {
   NN_CHECK(b && tau && certified && bound && fail_index, NNSDP_ERR_ARG, "NULL argument");
   NN_CHECK(b->ring > 0 && !b->dense && !b->packed, NNSDP_ERR_ARG,
            "nnsdp_batch_certify needs a batch in NNSDP_FORMAT_BLOCKS with ring_queries > 0");
@@ -2507,6 +2504,13 @@ extern "C" int32_t nnsdp_batch_certify_ex(nnsdp_batch* b, const double* tau, int
   NN_CHECK(b->prepared, NNSDP_ERR_STATE, "nnsdp_batch_certify before nnsdp_batch_prepare");
   for (int64_t q = 0; q < b->Q; ++q)
     NN_CHECK(std::isfinite(tau[q * tau_stride]), NNSDP_ERR_ARG, "tau of query %lld is not finite", (long long)q);
+  return NNSDP_OK;
+}
+
+// The factorisation of tau' I - Z for every query, tau' from tau[q * tau_stride].  A tau of -inf (nnsdp_batch_certify_gamma
+// with an infinite assembly error) runs no factorisation: the query is not certified, bound = +inf, lower = -inf.
+static int32_t certify_run(nnsdp_batch* b, const double* tau, int64_t tau_stride, int32_t* certified, double* bound,
+                           int64_t* fail_index, double* min_pivot, double* lower) {
   NN_CUDA(cudaSetDevice(b->dev));
   const Shape& sh = b->net->sh;
   if (b->chol.empty()) {
@@ -2541,12 +2545,19 @@ extern "C" int32_t nnsdp_batch_certify_ex(nnsdp_batch* b, const double* tau, int
     NN_CUDA(cudaMemcpyAsync(hstats.data(), dstats.p, (size_t)nq * 24, cudaMemcpyDeviceToHost, b->st));
     NN_CUDA(cudaStreamSynchronize(b->st));
     for (int i = 0; i < nq; ++i) {
-      htaup[i] = certify_shift(tau[(q0 + i) * tau_stride], sh.Zdim, hstats[3 * i], hstats[3 * i + 1], hstats[3 * i + 2],
-                               &bound[q0 + i]);
-      hlower[i] = certify_lower(htaup[i], sh.Zdim, hstats[3 * i + 2]);
-      hfailed[i] = 0;
+      const double t = tau[(q0 + i) * tau_stride];
       hfidx[i] = -1;
       hminp[i] = INFINITY;
+      if (!std::isfinite(t)) {  // marked failed: the kernels skip the query
+        htaup[i] = 0.0;
+        bound[q0 + i] = INFINITY;
+        hlower[i] = -INFINITY;
+        hfailed[i] = 1;
+        continue;
+      }
+      htaup[i] = certify_shift(t, sh.Zdim, hstats[3 * i], hstats[3 * i + 1], hstats[3 * i + 2], &bound[q0 + i]);
+      hlower[i] = certify_lower(htaup[i], sh.Zdim, hstats[3 * i + 2]);
+      hfailed[i] = 0;
     }
     NN_CUDA(cudaMemcpyAsync(dtaup.p, htaup.data(), (size_t)nq * 8, cudaMemcpyHostToDevice, b->st));
     NN_CUDA(cudaMemcpyAsync(dfailed.p, hfailed.data(), (size_t)nq * 4, cudaMemcpyHostToDevice, b->st));
@@ -2573,6 +2584,134 @@ extern "C" int32_t nnsdp_batch_certify_ex(nnsdp_batch* b, const double* tau, int
       // an infinite or NaN failing pivot means an overflow or a non-finite Z: the failure then proves nothing
       if (lower) lower[q0 + i] = hfailed[i] && std::isfinite(hminp[i]) ? hlower[i] : -INFINITY;
     }
+  }
+  return NNSDP_OK;
+}
+
+extern "C" int32_t nnsdp_batch_certify(nnsdp_batch* b, const double* tau, int64_t tau_stride, int32_t* certified,
+                                       double* bound, int64_t* fail_index, double* min_pivot) {
+  return nnsdp_batch_certify_ex(b, tau, tau_stride, certified, bound, fail_index, min_pivot, nullptr);
+}
+
+extern "C" int32_t nnsdp_batch_certify_ex(nnsdp_batch* b, const double* tau, int64_t tau_stride, int32_t* certified,
+                                          double* bound, int64_t* fail_index, double* min_pivot, double* lower) {
+  NN_TRY(certify_check(b, tau, tau_stride, certified, bound, fail_index));
+  return certify_run(b, tau, tau_stride, certified, bound, fail_index, min_pivot, lower);
+}
+
+
+// ---------------------------------------------------------------------------------------------
+// The certificate for the exact Z(gamma) (DESIGN.md section 9): e_q >= ||Z_dev - Z(gamma)||_inf from the entrywise
+// rounding bound of section 2, then the factorisation at tau - e_q.
+// ---------------------------------------------------------------------------------------------
+namespace {
+
+// An upper bound of N[r, c] = (monomials of Z[r, c]) + CHAIN + 2 over all entries (oracle/exact_z.py counts every
+// input as one factor, zeros included, and the constant 2 as none).  Per class of entry, with beta' = min(beta, acdim-1):
+//   Z[a, a]                 n1 + 4 acdim + output part
+//   affine entries          x_1: 2 + t1 + 3 n[1];  neuron rows: 4 + (2 + 4 beta') + (3 n[b+1] | tK)
+//   diagonal-block entries  Gram n[b+1] + F(r,c) + F(c,r) 2 (2 + 4 beta') + band 1 + 2 beta' (+ Zin, S11 | + W_K'S22W_K)
+//   other entries           2 (2 + 4 beta') + 1 + 2 beta' + S12 W_K
+int64_t zerr_count_max(const Shape& sh, int64_t beta, int32_t out_kind) {
+  const int K = sh.K;
+  const int64_t n1 = sh.n[0], no = sh.n[K], ac = sh.acdim, bt = std::min<int64_t>(beta, std::max<int64_t>(ac - 1, 0));
+  // monomials of one entry of S11, S12, S13, S22 (per row: s22r), S23, S33 (src/Qc/output.jl:52-98)
+  int64_t s11 = 0, s12 = 0, s13 = 0, s22r = 0, s23 = 0, s33 = 0;
+  if (out_kind == NNSDP_OUT_SAFETY) s11 = s12 = s13 = s23 = s33 = 1, s22r = no;
+  if (out_kind == NNSDP_OUT_HPLANE) s23 = 1, s33 = 1;
+  if (out_kind == NNSDP_OUT_CIRCLE) s22r = 1, s23 = 1, s33 = no + 1;
+  if (out_kind == NNSDP_OUT_ELLIPSOID) s22r = no * no, s23 = no, s33 = no + 1;
+  const int64_t f = 2 * (2 + 4 * bt), band = 1 + 2 * bt;
+  int64_t m = n1 + 4 * ac + no * s22r + 2 * no * s23 + s33;                       // Z[a, a]
+  m = std::max(m, 2 + no * s12 + s13 + 3 * sh.n[1]);                              // affine entries of x_1
+  m = std::max(m, f + band + no * s12);                                           // off-diagonal blocks
+  for (int b = 1; b <= K - 1; ++b)                                                // affine entries of neuron rows
+    m = std::max(m, 4 + 2 + 4 * bt + (b <= K - 2 ? 3 * sh.n[b + 1] : no * (s22r + s23)));
+  for (int b = 0; b <= K - 1; ++b)                                                // diagonal blocks
+    m = std::max(m, (b <= K - 2 ? sh.n[b + 1] : 0) + f + band + (b == 0 ? 1 + s11 : 0) + (b == K - 1 ? no * s22r : 0));
+  return m + 4 + 2;
+}
+
+// x + y and x - y rounded up / down (TwoSum: the rounding error of fl(x + y) is exact)
+double add_ru(double x, double y) {
+  const double s = x + y;
+  if (!std::isfinite(s)) return s;
+  const double bb = s - x, e = (x - (s - bb)) + (y - bb);
+  return e > 0 ? std::nextafter(s, INFINITY) : s;
+}
+double sub_rd(double x, double y) {
+  const double s = x - y;
+  if (!std::isfinite(s)) return s;
+  const double bb = s - x, e = (x - (s - bb)) + (-y - bb);
+  return e < 0 ? std::nextafter(s, -INFINITY) : s;
+}
+
+// e_q into err[Q] (host), the row sums s_q into rows[Zdim x Q] (host, may be null)
+int32_t assembly_error_run(nnsdp_batch* b, double* err, double* rows) {
+  NN_CUDA(cudaSetDevice(b->dev));
+  const Shape& sh = b->net->sh;
+  const NetPerDev& nd = *b->nd;
+  const int64_t Q = b->Q, nr = sh.acdim + sh.n_out();
+  const int64_t npart = (sh.acdim + ZERR_THREADS - 1) / ZERR_THREADS;
+  NN_TRY(b->ze_netv.ensure((size_t)(2 * nr + 1) * 8));
+  NN_TRY(b->ze_g.ensure((size_t)sh.acdim * Q * 8));
+  NN_TRY(b->ze_rows.ensure((size_t)sh.Zdim * Q * 8));
+  NN_TRY(b->ze_part.ensure((size_t)4 * npart * Q * 8));
+  NN_TRY(b->ze_io.ensure((size_t)4 * Q * 8));
+  NN_TRY(b->ze_err.ensure((size_t)Q * 8));
+  const int64_t nmax = zerr_count_max(sh, b->beta, b->bd.out_kind);
+  const double u = 0x1p-52, nu = up((double)nmax * u);
+  const double gN = up(nu / dn(1.0 - nu));                                  // gamma_Nmax
+  const double uf = up(std::ldexp((double)sh.Zdim * (double)nmax, -1074));  // Zdim Nmax 2^-1074
+  std::vector<const double*> wt(sh.K);
+  for (int k = 0; k < sh.K; ++k) wt[k] = nd.Wt[k].as<double>();
+  launch_zerr_net(nd.nd, b->ze_netv.as<double>(), b->st);
+  launch_zerr_query(nd.nd, b->bd, sh, wt.data(), b->net->ldT.data(), b->ze_netv.as<double>(), b->ze_g.as<double>(),
+                    b->ze_rows.as<double>(), b->ze_part.as<double>(), b->ze_io.as<double>(), gN, uf,
+                    b->ze_err.as<double>(), b->st);
+  NN_CUDA(cudaGetLastError());
+  NN_CUDA(cudaMemcpyAsync(err, b->ze_err.p, (size_t)Q * 8, cudaMemcpyDeviceToHost, b->st));
+  if (rows) NN_CUDA(cudaMemcpyAsync(rows, b->ze_rows.p, (size_t)sh.Zdim * Q * 8, cudaMemcpyDeviceToHost, b->st));
+  NN_CUDA(cudaStreamSynchronize(b->st));
+  return NNSDP_OK;
+}
+
+}  // namespace
+
+extern "C" int32_t nnsdp_assembly_error_nmax(int64_t K, const int64_t* xdims, int64_t beta, int32_t out_kind,
+                                             int64_t* nmax) {
+  NN_CHECK(nmax != nullptr, NNSDP_ERR_ARG, "NULL argument");
+  NN_CHECK(out_kind >= NNSDP_OUT_SAFETY && out_kind <= NNSDP_OUT_ELLIPSOID, NNSDP_ERR_ARG, "unrecognized out_kind %d",
+           (int)out_kind);
+  Shape sh;
+  NN_TRY(shape_from_xdims(K, xdims, &sh));
+  NN_CHECK(beta >= 0, NNSDP_ERR_ARG, "beta must be >= 0");
+  *nmax = zerr_count_max(sh, beta, out_kind);
+  return NNSDP_OK;
+}
+
+extern "C" int32_t nnsdp_batch_assembly_error(nnsdp_batch* b, double* err, double* abs_rowsum) {
+  NN_CHECK(b && err, NNSDP_ERR_ARG, "NULL argument");
+  NN_CHECK(b->ring > 0, NNSDP_ERR_ARG, "nnsdp_batch_assembly_error needs a batch with ring_queries > 0");
+  NN_CHECK(b->prepared, NNSDP_ERR_STATE, "nnsdp_batch_assembly_error before nnsdp_batch_prepare");
+  return assembly_error_run(b, err, abs_rowsum);
+}
+
+extern "C" int32_t nnsdp_batch_certify_gamma(nnsdp_batch* b, const double* tau, int64_t tau_stride, int32_t* certified,
+                                             double* bound, int64_t* fail_index, double* min_pivot, double* lower,
+                                             double* assembly_err) {
+  NN_TRY(certify_check(b, tau, tau_stride, certified, bound, fail_index));
+  const int64_t Q = b->Q;
+  std::vector<double> e(Q), taud(Q), low(Q);
+  NN_TRY(assembly_error_run(b, e.data(), nullptr));
+  for (int64_t q = 0; q < Q; ++q)  // largest double <= tau - e_q; -inf when e_q is infinite
+    taud[q] = std::isfinite(e[q]) ? sub_rd(tau[q * tau_stride], e[q]) : -INFINITY;
+  NN_TRY(certify_run(b, taud.data(), 1, certified, bound, fail_index, min_pivot, low.data()));
+  for (int64_t q = 0; q < Q; ++q) {
+    // certified: bound_dev <= tau - e_q exactly, so the smallest double >= bound_dev + e_q is still <= tau
+    bound[q] = std::isfinite(e[q]) ? add_ru(bound[q], e[q]) : INFINITY;
+    if (lower) lower[q] = std::isfinite(low[q]) && std::isfinite(e[q]) ? sub_rd(low[q], e[q]) : -INFINITY;
+    if (assembly_err) assembly_err[q] = e[q];
   }
   return NNSDP_OK;
 }

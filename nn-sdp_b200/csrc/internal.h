@@ -486,6 +486,15 @@ int launch_chol_front_init(double* ring, long long per, const CholFront& f, cons
 int launch_chol_panel(double* ring, long long per, const CholFront& f, int j0, int w, int nq, int* failed,
                       long long* fail_index, double* min_pivot, cudaStream_t st);
 
+// assembly-error bound (kernels_zerr.cu).  netv: 2 (acdim + n_out) + 1 doubles, per net (row sums of |W|, row maxima,
+// the largest |W|, |b|).  Per query: g (acdim), rows (Zdim: s[r] >= sum_c abs[r, c]), part (4 per CTA of the neuron
+// kernel), io (4), err (1) = gN max_r s[r] + uf F_q, rounded up (+inf when something is not finite).
+int launch_zerr_net(const NetDev& net, double* netv, cudaStream_t st);
+int launch_zerr_query(const NetDev& net, const BatchDev& b, const Shape& sh, const double* const* Wt, const int* ldT,
+                      const double* netv, double* g, double* rows, double* part, double* io, double gN, double uf,
+                      double* err, cudaStream_t st);
+constexpr int ZERR_THREADS = 256;  // neurons per CTA of the neuron kernel (the number of row-a partials follows)
+
 // band jobs (in-place band of the DIAG ranges, BAND cells of packed records) for queries [q0, q0+nq); after the fill kernel
 int launch_emit_band(const NetDev& net, const BatchDev& b, const GramDev& g, const BandDev* bands, int nbands,
                      int max_m, long long per_query, int q0, int nq, double* out, cudaStream_t st);

@@ -306,9 +306,11 @@ end
 # Sound form of the same acceptance test (nnsdp_batch_certify): a Cholesky factorisation of τ'I - Z(γ) along the
 # cliques with a margin for its rounding error.  Returns (certified, bound, lower): certified == true PROVES
 # eigmax(Z) <= bound <= τ for the FP64 Z the library assembles; false proves eigmax(Z) >= lower instead (from the
-# failed factorisation, nnsdp_batch_certify_ex; lower = -Inf when certified).
+# failed factorisation, nnsdp_batch_certify_ex; lower = -Inf when certified).  of_gamma = true makes both statements
+# about the exact Z(γ) of the same inputs instead (nnsdp_batch_certify_gamma: the factorisation at τ minus a bound on
+# the assembly's rounding error, see assemblyErrorB200).
 function eigmaxLeB200(net::DeviceNet, β::Int, qc_input, qc_out, qc_bounded, qc_sector, γin, γacs, γout = Float64[];
-                      τ::Float64 = 1e-4)
+                      τ::Float64 = 1e-4, of_gamma::Bool = false)
   keep = Any[]
   qi = Ref(query_inputs(qc_input, qc_out, qc_bounded, qc_sector, Vector{Float64}(γin),
                         [Vector{Float64}(g) for g in γacs], Vector{Float64}(γout), keep))
@@ -316,17 +318,45 @@ function eigmaxLeB200(net::DeviceNet, β::Int, qc_input, qc_out, qc_bounded, qc_
   check(ccall((:nnsdp_batch_create, LIB), Int32,
               (Ptr{Cvoid}, Int32, Ptr{Cvoid}, Int64, Int64, Int64, Int32, Ptr{Ptr{Cvoid}}),
               net.ctx.h, 0, net.h, β, 1, 1, 0, h))
-  tau, cert, bound, fidx, lower = [τ], zeros(Int32, 1), zeros(1), zeros(Int64, 1), zeros(1)
+  tau, cert, bound, fidx, lower, err = [τ], zeros(Int32, 1), zeros(1), zeros(Int64, 1), zeros(1), zeros(1)
   try
     GC.@preserve keep check(ccall((:nnsdp_batch_set_inputs, LIB), Int32, (Ptr{Cvoid}, Int64, Ptr{QueryInputs}), h[], 1, qi))
     check(ccall((:nnsdp_batch_prepare, LIB), Int32, (Ptr{Cvoid},), h[]))
-    check(ccall((:nnsdp_batch_certify_ex, LIB), Int32,
-                (Ptr{Cvoid}, Ptr{Float64}, Int64, Ptr{Int32}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}),
-                h[], tau, 0, cert, bound, fidx, C_NULL, lower))
+    if of_gamma
+      check(ccall((:nnsdp_batch_certify_gamma, LIB), Int32,
+                  (Ptr{Cvoid}, Ptr{Float64}, Int64, Ptr{Int32}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}, Ptr{Float64},
+                   Ptr{Float64}),
+                  h[], tau, 0, cert, bound, fidx, C_NULL, lower, err))
+    else
+      check(ccall((:nnsdp_batch_certify_ex, LIB), Int32,
+                  (Ptr{Cvoid}, Ptr{Float64}, Int64, Ptr{Int32}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}),
+                  h[], tau, 0, cert, bound, fidx, C_NULL, lower))
+    end
   finally
     ccall((:nnsdp_batch_destroy, LIB), Int32, (Ptr{Cvoid},), h[])
   end
   return cert[1] == 1, bound[1], lower[1]
+end
+
+# e ≥ ‖Z_dev - Z(γ)‖∞ (nnsdp_batch_assembly_error): how far the FP64 Z the library assembles can be from the exact
+# Z(γ) of the same inputs, QC bounds as computed by the library; so eigmax(Z(γ)) lies within e of eigmax(Z_dev).
+function assemblyErrorB200(net::DeviceNet, β::Int, qc_input, qc_out, qc_bounded, qc_sector, γin, γacs, γout = Float64[])
+  keep = Any[]
+  qi = Ref(query_inputs(qc_input, qc_out, qc_bounded, qc_sector, Vector{Float64}(γin),
+                        [Vector{Float64}(g) for g in γacs], Vector{Float64}(γout), keep))
+  h = Ref{Ptr{Cvoid}}(C_NULL)
+  check(ccall((:nnsdp_batch_create, LIB), Int32,
+              (Ptr{Cvoid}, Int32, Ptr{Cvoid}, Int64, Int64, Int64, Int32, Ptr{Ptr{Cvoid}}),
+              net.ctx.h, 0, net.h, β, 1, 1, 0, h))
+  err = zeros(1)
+  try
+    GC.@preserve keep check(ccall((:nnsdp_batch_set_inputs, LIB), Int32, (Ptr{Cvoid}, Int64, Ptr{QueryInputs}), h[], 1, qi))
+    check(ccall((:nnsdp_batch_prepare, LIB), Int32, (Ptr{Cvoid},), h[]))
+    check(ccall((:nnsdp_batch_assembly_error, LIB), Int32, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}), h[], err, C_NULL))
+  finally
+    ccall((:nnsdp_batch_destroy, LIB), Int32, (Ptr{Cvoid},), h[])
+  end
+  return err[1]
 end
 
 # ---- vnnlib property -> batched safety queries (experiments/vnnlib_utils.jl:18-56) -------------------

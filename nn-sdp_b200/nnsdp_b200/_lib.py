@@ -106,6 +106,9 @@ PROTOTYPES = {
     "nnsdp_batch_certify": (c_i32, [c_vp, c_dp, c_i64, C.POINTER(c_i32), c_dp, c_i64p, c_dp]),
     "nnsdp_batch_certify_ex": (c_i32, [c_vp, c_dp, c_i64, C.POINTER(c_i32), c_dp, c_i64p, c_dp, c_dp]),
     "nnsdp_certify_plan": (c_i32, [c_i64, c_i64p, c_i64, c_i64, c_i64p, c_i64p]),
+    "nnsdp_batch_assembly_error": (c_i32, [c_vp, c_dp, c_dp]),
+    "nnsdp_assembly_error_nmax": (c_i32, [c_i64, c_i64p, c_i64, c_i32, c_i64p]),
+    "nnsdp_batch_certify_gamma": (c_i32, [c_vp, c_dp, c_i64, C.POINTER(c_i32), c_dp, c_i64p, c_dp, c_dp, c_dp]),
     "nnsdp_affine_create": (c_i32, [c_vp, c_vp, c_i64, C.POINTER(QueryInputs), c_i64, C.POINTER(c_vp), C.POINTER(AffineSizes)]),
     "nnsdp_affine_get": (c_i32, [c_vp, c_i64p, c_i64p, c_dp, c_i64p, c_i64p, c_dp]),
     "nnsdp_affine_destroy": (c_i32, [c_vp]),

@@ -179,6 +179,15 @@ def plan_panel(xdims: Sequence[int], beta: int, dense: int = 0) -> np.ndarray:
 CERTIFY_PLAN_FIELDS = ("out_off", "n", "npriv", "g0", "lead", "tail")
 
 
+def assembly_error_nmax(xdims: Sequence[int], beta: int, out_kind: int) -> int:
+    """Nmax of Batch.assembly_error (nnsdp_assembly_error_nmax): an upper bound of the monomial count + 6 of every
+    entry of Z for these layer widths, beta and output kind (host only)."""
+    xd = np.ascontiguousarray(xdims, dtype=np.int64)
+    n = L.c_i64(0)
+    L.check(L.lib.nnsdp_assembly_error_nmax(len(xd) - 1, xd.ctypes.data_as(L.c_i64p), beta, out_kind, C.byref(n)))
+    return int(n.value)
+
+
 def certify_plan(xdims: Sequence[int], beta: int) -> np.ndarray:
     """The elimination plan of Batch.certify as an (nfronts, 6) int64 array (columns: CERTIFY_PLAN_FIELDS).  Raises
     NnsdpError(ERR_ASSERT) if a layout fact of the multifrontal factorisation does not hold.  Host only."""
@@ -600,15 +609,44 @@ class Batch:
                                              fidx.ctypes.data_as(L.c_i64p), _dp(minp), _dp(lo) if lower else None))
         return (cert, bound, fidx, minp, lo) if lower else (cert, bound, fidx, minp)
 
+    def assembly_error(self, rowsums: bool = False):
+        """e_q >= ||Z_dev - Z(gamma)||_inf for every query (nnsdp_batch_assembly_error): the distance between the FP64 Z
+        the library emits and the exact Z(gamma) of the same inputs (the QC bounds as the batch holds them); needs
+        bounds + prepare.  +inf where an input or intermediate is not finite.  rowsums=True also returns s (Q x Zdim),
+        s[q, r] >= the sum over c of abs[r, c] (oracle/exact_z.py)."""
+        err = np.zeros(self.Q)
+        rows = np.zeros((self.Q, self.sz["Zdim"])) if rowsums else None
+        L.check(L.lib.nnsdp_batch_assembly_error(self._h, _dp(err), _dp(rows) if rowsums else None))
+        return (err, rows) if rowsums else err
+
+    def certify_gamma(self, tau, lower: bool = False):
+        """Sound certificate lambda_max(Z(gamma)_q) <= tau_q for the EXACT Z(gamma) (nnsdp_batch_certify_gamma): the
+        factorisation of certify at tau_q - e_q, e_q = assembly_error().  Returns what certify returns plus e_q last:
+        (certified, bound, fail_index, min_pivot[, lower], err).  certified[q] = 1 proves
+        lambda_max(Z(gamma)_q) <= bound[q] <= tau_q; lower (lower=True) proves lambda_max(Z(gamma)_q) >= lower[q] for a
+        query that was not certified (-inf when nothing is proven)."""
+        t = np.ascontiguousarray(np.atleast_1d(np.asarray(tau, dtype=np.float64)))
+        if t.size not in (1, self.Q):
+            raise ValueError(f"tau has {t.size} values for {self.Q} queries")
+        cert = np.zeros(self.Q, dtype=np.int32)
+        bound, minp, lo, err = (np.zeros(self.Q) for _ in range(4))
+        fidx = np.zeros(self.Q, dtype=np.int64)
+        L.check(L.lib.nnsdp_batch_certify_gamma(self._h, _dp(t), 0 if t.size == 1 else 1,
+                                                cert.ctypes.data_as(C.POINTER(L.c_i32)), _dp(bound),
+                                                fidx.ctypes.data_as(L.c_i64p), _dp(minp), _dp(lo) if lower else None,
+                                                _dp(err)))
+        return (cert, bound, fidx, minp, lo, err) if lower else (cert, bound, fidx, minp, err)
+
     def lambda_max_bracket(self, max_iters: int = 300, tol: float = 1e-10, rel: float = 1e-9, growth: float = 10.0,
-                           max_tries: int = 12, scale=None):
+                           max_tries: int = 12, scale=None, of_gamma: bool = False):
         """A sound interval lo <= lambda_max(Z_q) <= hi for every query, both ends proven by a factorisation of
         fl(tau' I - Z): hi is the bound of a certified call, lo the lower bound of a failed one (certify(lower=True)).
         The Lanczos Ritz value r only places the tries: it is not a bound (its rounding error may put it above
         lambda_max).  The first try is tau = r; then a query still without hi tries r + rel * scale * growth^t, one
         still without lo tries r - rel * scale * growth^t, t = 0, 1, ..., at most max_tries calls in all.  An end no try
         proves stays -inf / inf.  scale (per query or scalar) defaults to max(|r|, resid).  Returns (lo, hi, certified),
-        certified = 1 where hi is finite."""
+        certified = 1 where hi is finite.  of_gamma=True brackets lambda_max of the exact Z(gamma) instead, every try
+        through certify_gamma (the interval then holds the assembly error e_q on both sides)."""
         r, _, resid, _ = self.lambda_max(max_iters=max_iters, tol=tol, full=True)
         s = np.maximum(np.abs(r), resid) if scale is None else np.broadcast_to(np.asarray(scale, dtype=float), r.shape)
         s = np.maximum(s, np.finfo(float).tiny)
@@ -617,7 +655,10 @@ class Batch:
         tau = r.copy()
         step = rel * s
         for _ in range(max_tries):
-            cert, bound, _, _, low = self.certify(tau, lower=True)
+            if of_gamma:
+                cert, bound, _, _, low, _ = self.certify_gamma(tau, lower=True)
+            else:
+                cert, bound, _, _, low = self.certify(tau, lower=True)
             ok = cert == 1
             hi[ok] = np.minimum(hi[ok], bound[ok])
             lo[~ok] = np.maximum(lo[~ok], low[~ok])
