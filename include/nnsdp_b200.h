@@ -293,6 +293,15 @@ int32_t nnsdp_batch_bounds(nnsdp_batch* batch);
 #define NNSDP_BOUNDS_CROWN 1
 int32_t nnsdp_batch_bounds_crown(nnsdp_batch* batch);
 int32_t nnsdp_batch_set_bounds_method(nnsdp_batch* batch, int32_t method);
+/* Introspection of the CROWN pass (off by default; nothing is allocated or copied while off).  With keeping on, every
+ * CROWN pass of the batch (nnsdp_batch_bounds_crown, or nnsdp_batch_run with NNSDP_BOUNDS_CROWN) also keeps the
+ * pre-activation bounds y_0 .. y_{K-1} it computed, from which each later layer's relaxation was built.
+ * nnsdp_batch_get_crown_preact copies them out (either pointer may be NULL; blocking): prel / preu are Q x P, row q =
+ * [y_0; ...; y_{K-1}] of query q, P = xtot - n_in.  y_0 is the interval-arithmetic layer, y_{K-1} the output layer
+ * before the min/max of x_K.  NNSDP_ERR_STATE while keeping is off or before a CROWN pass on the current inputs.
+ * Turning keeping off releases the copy. */
+int32_t nnsdp_batch_keep_crown_preact(nnsdp_batch* batch, int32_t on);
+int32_t nnsdp_batch_get_crown_preact(nnsdp_batch* batch, double* prel, double* preu);
 /* QC diagonals, band multipliers, affine column (all queries of the batch). */
 int32_t nnsdp_batch_prepare(nnsdp_batch* batch);
 /* Gram contractions + block emission of queries [q0, q0+nq) into ring slots

@@ -251,6 +251,10 @@ struct nnsdp_batch {
   DevBuf d11, Md, T0, Bt, u, aff, part, act, cnt, Z11, Z1K, U;
   DevBuf gram, ringbuf, flags;
   DevBuf cr_rowsA, cr_rowsB, cr_bias, cr_prel, cr_preu, cr_du, cr_bu, cr_dl;  // CROWN work buffers (kept when small)
+  // CROWN pre-activation bounds y_0 .. y_{K-1} of every query (Q x (xtot - n_in)), copied out of cr_prel / cr_preu
+  // when keep_preact is on (nnsdp_batch_keep_crown_preact); valid after a CROWN pass on the current inputs
+  DevBuf cr_keep_l, cr_keep_u;
+  bool keep_preact = false, preact_valid = false;
   BatchDev bd{};
   GramDev gd{};
   PlanDev pd{};
@@ -305,7 +309,8 @@ struct nnsdp_batch {
     return {&d_bands, &d_tmaps, &d_tmap_ok, &d_tiles, &d_strips, &d_bulk, &d_mats, &d_panel, &d_goff, &d_ldG, &d_chol, &ze_netv, &ze_g, &ze_rows, &ze_part, &ze_io, &ze_err, &x1min, &x1max, &ymin, &ymax, &smin, &smax,
             &gin, &gbnd, &gsec, &outS, &outvec, &outinvP, &gout, &xmin, &xmax, &acxmin, &acxmax,
             &smin_c, &smax_c, &d11, &Md, &T0, &Bt, &u, &aff, &part, &act, &cnt, &Z11, &Z1K, &U,
-            &gram, &ringbuf, &flags, &cr_rowsA, &cr_rowsB, &cr_bias, &cr_prel, &cr_preu, &cr_du, &cr_bu, &cr_dl};
+            &gram, &ringbuf, &flags, &cr_rowsA, &cr_rowsB, &cr_bias, &cr_prel, &cr_preu, &cr_du, &cr_bu, &cr_dl,
+            &cr_keep_l, &cr_keep_u};
   }
 };
 
@@ -381,7 +386,7 @@ int32_t check_flags(nnsdp_batch* b, const char* where) {
 extern "C" {
 
 const char* nnsdp_last_error(void) { return g_err.c_str(); }
-int32_t nnsdp_version(void) { return 103; }
+int32_t nnsdp_version(void) { return 104; }
 
 int32_t nnsdp_device_count(int32_t* count) {
   NN_CHECK(count != nullptr, NNSDP_ERR_ARG, "count is NULL");
@@ -991,6 +996,7 @@ int32_t nnsdp_batch_set_inputs(nnsdp_batch* b, int64_t Q, const nnsdp_query_inpu
   cudaStream_t st = b->st;
   b->have_inputs = false;
   b->bounds_done = b->prepared = false;
+  b->preact_valid = false;
   b->Q = Q;
   bd.Q = (int)Q;
   bd.beta = (int)b->beta;
@@ -1087,6 +1093,7 @@ int32_t nnsdp_batch_bounds(nnsdp_batch* b) {
   const int Q = (int)b->Q;
   double* xmin = b->xmin.as<double>();
   double* xmax = b->xmax.as<double>();
+  b->preact_valid = false;  // these bounds are not the CROWN ones any more
   b->span_begin(ST_BOUNDS, b->st);
   int launches = 0;
   int max_out = 0;
@@ -2041,6 +2048,11 @@ int32_t crown_bounds_device(nnsdp_batch* b) {
   NN_TRY(rowsB.ensure((size_t)2 * Qc * rows_cap * ld * 8));
   NN_TRY(bias.ensure((size_t)2 * Qc * rows_cap * 8));
   for (DevBuf* x : {&prel, &preu, &du, &bu, &dl}) NN_TRY(x->ensure((size_t)Qc * P * 8));
+  b->preact_valid = false;
+  if (b->keep_preact) {
+    NN_TRY(b->cr_keep_l.ensure((size_t)b->Q * P * 8));
+    NN_TRY(b->cr_keep_u.ensure((size_t)b->Q * P * 8));
+  }
   cudaStream_t st = b->st;
   double* xmin = b->xmin.as<double>();
   double* xmax = b->xmax.as<double>();
@@ -2116,6 +2128,12 @@ int32_t crown_bounds_device(nnsdp_batch* b) {
         launches += launch_crown_params(prel.as<double>() + poff(t), preu.as<double>() + poff(t), P, nrows, nq,
                                         du.as<double>() + poff(t), bu.as<double>() + poff(t),
                                         dl.as<double>() + poff(t), st);
+    }
+    if (b->keep_preact) {  // the chunk's y_0 .. y_{K-1}: nq rows of P, contiguous on both sides
+      NN_CUDA(cudaMemcpyAsync(b->cr_keep_l.as<double>() + q0 * P, prel.as<double>(), (size_t)nq * P * 8,
+                              cudaMemcpyDeviceToDevice, st));
+      NN_CUDA(cudaMemcpyAsync(b->cr_keep_u.as<double>() + q0 * P, preu.as<double>(), (size_t)nq * P * 8,
+                              cudaMemcpyDeviceToDevice, st));
     }
     // x_{k+1} = relu(y_k), k = 0 .. K-2: the output of the (k+1)-layer prefix followed by an identity layer.  Its
     // chains are row scalings of the chains of y_k that are already finished (see crown_post_kernel): one launch.
@@ -2202,10 +2220,35 @@ int32_t crown_bounds_device(nnsdp_batch* b) {
   NN_CUDA(cudaGetLastError());
   NN_CUDA(cudaStreamSynchronize(st));  // the temporary buffers are released on return
   b->bounds_done = true;
+  b->preact_valid = b->keep_preact;
   return NNSDP_OK;
 }
 
 }  // namespace
+
+extern "C" int32_t nnsdp_batch_keep_crown_preact(nnsdp_batch* b, int32_t on) {
+  NN_CHECK(b != nullptr, NNSDP_ERR_ARG, "batch is NULL");
+  b->keep_preact = on != 0;
+  if (!b->keep_preact) {
+    NN_CUDA(cudaSetDevice(b->dev));
+    b->cr_keep_l.release();
+    b->cr_keep_u.release();
+    b->preact_valid = false;
+  }
+  return NNSDP_OK;
+}
+
+extern "C" int32_t nnsdp_batch_get_crown_preact(nnsdp_batch* b, double* prel, double* preu) {
+  NN_CHECK(b != nullptr, NNSDP_ERR_ARG, "batch is NULL");
+  NN_CHECK(b->keep_preact, NNSDP_ERR_STATE, "keeping the CROWN pre-activation bounds is off");
+  NN_CHECK(b->preact_valid, NNSDP_ERR_STATE, "no CROWN pass on the current inputs since keeping was turned on");
+  NN_CUDA(cudaSetDevice(b->dev));
+  const size_t bytes = (size_t)b->Q * (b->net->sh.xtot - b->net->sh.n_in()) * 8;
+  if (prel) NN_CUDA(cudaMemcpyAsync(prel, b->cr_keep_l.p, bytes, cudaMemcpyDeviceToHost, b->st));
+  if (preu) NN_CUDA(cudaMemcpyAsync(preu, b->cr_keep_u.p, bytes, cudaMemcpyDeviceToHost, b->st));
+  NN_CUDA(cudaStreamSynchronize(b->st));
+  return NNSDP_OK;
+}
 
 extern "C" int32_t nnsdp_batch_bounds_crown(nnsdp_batch* b) {
   NN_CHECK(b != nullptr, NNSDP_ERR_ARG, "batch is NULL");

@@ -97,6 +97,8 @@ PROTOTYPES = {
     "nnsdp_bounds_crown": (c_i32, [c_vp, c_vp, c_i64, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp]),
     "nnsdp_batch_bounds_crown": (c_i32, [c_vp]),
     "nnsdp_batch_set_bounds_method": (c_i32, [c_vp, c_i32]),
+    "nnsdp_batch_keep_crown_preact": (c_i32, [c_vp, c_i32]),
+    "nnsdp_batch_get_crown_preact": (c_i32, [c_vp, c_dp, c_dp]),
     "nnsdp_preact_from_x": (c_i32, [c_vp, c_vp, c_i64, c_dp, c_dp, c_dp, c_dp]),
     "nnsdp_sector_minmax": (c_i32, [c_vp, c_i64, c_dp, c_dp, c_dp, c_dp]),
     "nnsdp_assemble_blocks": (c_i32, [c_vp, c_vp, c_i64, c_i64, C.POINTER(QueryInputs), c_dp]),

@@ -547,6 +547,17 @@ class Batch:
     def set_bounds_method(self, method: str):
         L.check(L.lib.nnsdp_batch_set_bounds_method(self._h, {"ibp": 0, "crown": 1}[method]))
 
+    def keep_crown_preact(self, on: bool = True):
+        """nnsdp_batch_keep_crown_preact: keep the pre-activation bounds of every later CROWN pass (off by default)."""
+        L.check(L.lib.nnsdp_batch_keep_crown_preact(self._h, 1 if on else 0))
+
+    def get_crown_preact(self):
+        """(prel, preu), Q x (xtot - n_in): y_0 .. y_{K-1} of the last CROWN pass as the device computed them."""
+        P = self.sz["xtot"] - self.sz["n_in"]
+        lo, hi = np.empty((self.Q, P)), np.empty((self.Q, P))
+        L.check(L.lib.nnsdp_batch_get_crown_preact(self._h, _dp(lo), _dp(hi)))
+        return lo, hi
+
     def prepare(self):
         L.check(L.lib.nnsdp_batch_prepare(self._h))
 
