@@ -261,30 +261,42 @@ class ExactZ:
         b = (g * self.abs) * (1 + 2.0 ** -50) + self.N * 2.0 ** -1074
         return np.where(self.abs == 0, 0.0, b)
 
-    def error(self, Zrows):
-        """|Zrows − ref| (float64, rounded up) for FP64 values of the same rows."""
-        Zrows = np.asarray(Zrows, dtype=np.float64)
+    def error(self, Zrows, slack=None):
+        """|Zrows − ref| (float64, rounded up) for FP64 values of the same rows.  Zrows may also hold exact sums of
+        FP64 values (Fraction objects; long doubles in the extended mode); `slack` (float64 ≥ 0) is added to the error,
+        for a caller whose long double sums are themselves rounded."""
+        Zrows = _values(Zrows)
         if self.exact:
             d = np.abs(np.asarray(_frac(Zrows), dtype=object) - self.ref)
-            return _up(d, True)
-        d = np.abs(Zrows.astype(np.longdouble) - self.ref)
-        return _up(d * (1 + np.longdouble(2.0 ** -62)), False)
+            err = _up(d, True)
+        else:
+            d = np.abs(Zrows.astype(np.longdouble) - self.ref)
+            err = _up(d * (1 + np.longdouble(2.0 ** -62)), False)
+        if slack is not None:
+            err = np.nextafter(err + slack, np.inf)
+        return err
 
-    def check(self, Zrows):
-        """(ok mask, error / bound) of the entrywise criterion; ok is exact for the exact mode."""
-        Zrows = np.asarray(Zrows, dtype=np.float64)
-        err, bnd = self.error(Zrows), self.bound()
-        ok = np.where(self.abs == 0, Zrows == 0.0, err <= bnd)
-        if self.exact:                       # decide the entries close to the bound exactly
+    def check(self, Zrows, slack=None):
+        """(ok mask, error / bound) of the entrywise criterion; ok is exact for the exact mode (any array shape)."""
+        Zrows = _values(Zrows)
+        err, bnd = self.error(Zrows, slack), self.bound()
+        ok = np.where(self.abs == 0, Zrows == 0.0, err <= bnd).astype(bool)
+        if self.exact and slack is None:     # decide the entries close to the bound exactly
             close = ~ok | (err >= 0.5 * bnd)
-            for i, k in zip(*np.nonzero(close & (self.abs != 0))):
-                n = int(self.N[i, k])
+            for idx in zip(*np.nonzero(close & (self.abs != 0))):
+                n = int(self.N[idx])
                 gN = Fraction(n) * Fraction(U) / (1 - Fraction(n) * Fraction(U))
-                absx = self._abs_exact[i, k]
-                ok[i, k] = abs(Fraction(float(Zrows[i, k])) - self.ref[i, k]) <= gN * absx + n * ETA
+                absx = self._abs_exact[idx]
+                ok[idx] = abs(Fraction(Zrows[idx]) - self.ref[idx]) <= gN * absx + n * ETA
         with np.errstate(divide="ignore", invalid="ignore"):
             ratio = np.where(bnd > 0, err / bnd, np.where(Zrows == 0.0, 0.0, np.inf))
         return ok, ratio
+
+
+def _values(Z):
+    """FP64 values as float64; exact sums of them (Fraction objects, long doubles) as they are."""
+    Z = np.asarray(Z)
+    return Z if Z.dtype in (object, np.longdouble) else Z.astype(np.float64)
 
 
 def exact_z(net, beta: int, q, bounds, mode: str = "exact", rows: Optional[np.ndarray] = None) -> ExactZ:

@@ -135,9 +135,15 @@ def wide_range_case(xdims, beta, kind, seed):
     return net, q, bounds
 
 
-def assert_meets(R, Z, what=""):
-    ok, ratio = R.check(Z)
+def assert_meets(R, Z, what="", **kw):
+    """R (exact_z.ExactZ, or exact_affine.ExactAffine with Z the device's (var, ent, val) triplets) holds Z to the
+    entrywise criterion; the failure names the worst entry, for the hand-off as (variable, row, column)."""
+    ok, ratio = R.check(Z, **kw)
     if not ok.all():
+        if hasattr(R, "where"):
+            i = int(np.argmax(np.where(ok, 0, ratio)))
+            raise AssertionError(f"{what}: {int((~ok).sum())} coefficients break the bound; worst {R.where(i)}, "
+                                 f"|err| / bound = {ratio[i]:.3g}")
         i, c = np.unravel_index(np.argmax(np.where(ok, 0, ratio)), ok.shape)
         raise AssertionError(f"{what}: {int((~ok).sum())} entries break the bound; worst Z[{R.rows[i]},{c}] = "
                              f"{Z[i, c]!r}, |err| / bound = {ratio[i, c]:.3g}, abs = {R.abs[i, c]:.3g}, N = {R.N[i, c]}")
